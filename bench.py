@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SdBG-construction hot path (count -> seq2sdbg) on synthetic 150 bp reads, k=27.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of reads: canonical (k+1)-mer edge extraction, LSD
 radix sort, solid-edge counting + mercy bookkeeping, then seq2sdbg item extraction, radix sort and SdBG
@@ -9,6 +9,7 @@ emission from the device-resident solid edges.  `value` is whole-job edges/s wit
 in HBM; `e2e` is the same metric through the host-buffer C ABI (mhb_build_host: count -> device mercy edges -> seq2sdbg), H2D/D2H
 inside the timed region.  `--impl reference` times the unmodified reference's OpenMP path
 (oracle/_ref/megahit_core_ref count + seq2sdbg) on the host cores on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -194,6 +195,54 @@ def bind_to_gpu_numa(local: int):
     return "unbound"
 
 
+def _sorted_rows(rows):
+    """rows (n, W) int32 on the device in ascending lexicographic order of their uint32 words"""
+    import torch
+    key = rows.to(torch.int64) & 0xFFFFFFFF
+    idx = torch.arange(len(rows), device=rows.device)
+    for c in reversed(range(rows.shape[1])):
+        idx = idx[torch.sort(key[idx, c], stable=True).indices]
+    return rows[idx]
+
+
+def _sample(t, cap, seed):
+    """t itself when it has at most cap leading-dimension entries, else a fixed seeded sample of them (in order)"""
+    import torch
+    if len(t) <= cap:
+        return t
+    idx = np.sort(np.random.default_rng(seed).integers(0, len(t), size=cap))
+    return t[torch.from_numpy(idx).to(t.device)]
+
+
+def dump_outputs(d, plan, s2s, n_solid, n_mercy):
+    """What the last step handed its caller, as float64 (float32 for the SdBG bytes), under 51 MiB in all: the solid and
+    the mercy (k+1)-mer edges as rows of uint32 words (ascending; a seeded sample of at most 2^21 words each), the
+    `.counting` histogram, the SdBG bucket table {byte offset, items, tips, large multiplicities}, the SdBG totals
+    {bytes, items, tips, large, w counts[9], ones in last} and a seeded sample of at most 2^22 SdBG bytes."""
+    import torch
+    os.makedirs(d, exist_ok=True)
+    WE = plan.WE
+    edges = plan.edges[: (n_solid + n_mercy) * WE].view(-1, WE)
+    cap_rows = max(1, (1 << 21) // WE)
+    totals = s2s.totals[:14].cpu()
+    out = {
+        "solid_edges": _sample(_sorted_rows(edges[:n_solid]), cap_rows, 1),
+        "mercy_edges": _sample(_sorted_rows(edges[n_solid:]), cap_rows, 2),
+        "counting": plan.mul_hist,
+        "sdbg_bucket_table": s2s.table.view(-1, 4),
+        "sdbg_totals": totals,
+        "sdbg_bytes": _sample(s2s.bytes[: int(totals[0])], 1 << 22, 3),
+    }
+    for name, t in out.items():
+        if name == "sdbg_bytes":
+            a = t.cpu().numpy().astype(np.float32)
+        elif t.dtype == torch.int32:
+            a = t.cpu().numpy().view(np.uint32).astype(np.float64)
+        else:
+            a = t.cpu().numpy().astype(np.float64)
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
@@ -233,6 +282,7 @@ def ours(args):
     s2s = dev.S2sPlan(int((n_solid + n_mercy0) * 1.05) + 1024, k + 1, k, device)
 
     mercy_ev = []
+    last = {}
 
     def step(timed=False):
         # count (extract, partition/sort, solid edges, mercy marks) -> mercy edges -> seq2sdbg over solid + mercy edges:
@@ -244,6 +294,7 @@ def ours(args):
             e.record()
             mercy_ev.append(e)
         s2s.run(plan.edges, None, ns + nm, plan.WE, timed=timed, aux=plan.aux, n_aux=ns)
+        last.update(n_solid=ns, n_mercy=nm)
         return ns
 
     for _ in range(max(0, args.warmup - 1)):
@@ -270,6 +321,9 @@ def ours(args):
     clk = clocks.stop()
     ms_per_step = e0.elapsed_time(e1) / args.steps
     value = n_edges / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, plan, s2s, last["n_solid"], last["n_mercy"])
+        torch.cuda.empty_cache()  # the sort keys of the dump stay out of the way of the e2e arm's own allocations
 
     # stage split of the count stage
     ev = plan.events
@@ -398,7 +452,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--count-mode", default=None, choices=["sort", "hashed", "auto"],
                     help="count stage algorithm (default: $MHB_COUNT_MODE, else hashed where supported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (one GPU, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.impl == "reference":
         # exactly K timed + W warm-up steps; the per-step sample is sized so the whole run stays within minutes
         # (~8 s per 1 M reads on 8 host cores)

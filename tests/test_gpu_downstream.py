@@ -1,14 +1,15 @@
-"""GPU tests against the UNMODIFIED reference binary shipped to the GPU box as oracle/_ref/megahit_core_ref:
+"""GPU tests against the UNMODIFIED reference:
 
 * bench-scale parity: 1 M synthetic 150 bp reads (123 M edge records; thousands of radix tiles per pass, every CTA of
-  the persistent kernels busy) through the file-level commands, byte-compared with what the reference binary writes
-  for the same library (canonical streams, SURVEY.md 8c) - also with the count stage forced into >= 5 rounds and
-  through the fused build;
+  the persistent kernels busy) through the file-level commands, compared with the digests of what the reference binary
+  writes for the same library (canonical streams, SURVEY.md 8c; tests/golden/scale/, oracle/scale_golden.py) - also
+  with the count stage forced into >= 5 rounds and through the fused build;
 * downstream acceptance (north_star: "the reference's downstream assemble/local/iterate stages consume it unchanged"):
   the reference's `assemble` run on OUR `.sdbg.*` / `.sdbg_info` gives byte-identical contigs to the same command run
   on the reference-built graph (reader: sdbg/sdbg_raw_content.cpp:18-95, sdbg/sdbg_meta.cpp:24-48), and the reference's
   Python driver (src/megahit) completes a multi-k assembly with our `megahit_core` in its bin directory and produces the
-  same final contigs as with the reference core.
+  same final contigs as with the reference core.  These two run the reference binary itself (oracle/_ref/, which
+  build() compiles with `make -C oracle ref`).
 """
 import os
 import shutil
@@ -21,6 +22,7 @@ import pytest
 from conftest import GOLDEN, ROOT
 from megahit_b200 import formats as F
 from megahit_b200 import lib, synth
+from oracle import scale_golden as SG
 
 pytestmark = pytest.mark.gpu
 
@@ -31,8 +33,8 @@ OURS = os.path.join(ROOT, "megahit_b200", "bin", "megahit_core")
 
 def _need_ref():
     if not os.path.exists(REF):
-        pytest.fail("oracle/_ref/megahit_core_ref is missing: build it in the container (make -C oracle ref); it "
-                    "travels to the GPU box with the snapshot")
+        pytest.fail("oracle/_ref/megahit_core_ref is missing: build() compiles it (make -C oracle ref) from the "
+                    "reference sources")
 
 
 def _run(cmd, **kw):
@@ -48,26 +50,16 @@ def _ref_build(core, lib_prefix, p, k, m, threads=8, mercy=True):
           str(threads), "-k", str(k), "--kmer_from", "0", "--input_prefix", p] + (["--need_mercy"] if mercy else []))
 
 
-def _digests(p):
-    info, stream, table = F.canonical_sdbg(p)
-    return {"edges": F.sha256(F.canonical_edges(p).tobytes()), "cand": F.file_sha256(p + ".cand"),
-            "counting": F.file_sha256(p + ".counting"), "sdbg": F.sha256(stream), "k": info.k,
-            "wpt": info.words_per_tip_label, "items": int(table[:, 0].sum()), "tips": int(table[:, 1].sum()),
-            "large": int(table[:, 2].sum())}
+_digests = SG.count_sdbg_digests
 
 
 @pytest.fixture(scope="module")
 def big_case(tmp_path_factory):
-    """1 M x 150 bp, 30x, 1 % substitutions; the reference binary's output for it (k=27, m=2, mercy on)"""
-    _need_ref()
+    """1 M x 150 bp, 30x, 1 % substitutions; the digests of the reference binary's output for it (k=27, m=2, mercy on)"""
     d = tmp_path_factory.mktemp("big")
-    n_reads, L = 1_000_000, 150
-    b = synth.synth_reads(n_reads, L, 5 * n_reads, 0.01, seed=4242)
     libp = str(d / "reads.lib")
-    F.write_lib(libp, b, n_reads, n_reads * L, L)
-    rp = str(d / "ref")
-    _ref_build(REF, libp, rp, 27, 2, threads=min(32, os.cpu_count() or 8))
-    return {"lib": libp, "bin": b, "n_reads": n_reads, "ref": _digests(rp), "dir": d}
+    b = SG.big_lib(libp)
+    return {"lib": libp, "bin": b, "n_reads": len(b), "ref": SG.golden()["count_1m_k27_m2"], "dir": d}
 
 
 def test_bench_scale_file_level_matches_reference_binary(big_case):

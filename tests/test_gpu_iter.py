@@ -1,22 +1,21 @@
 """GPU tests of `iterate` (SURVEY.md 8f N2): the CUDA path through the C ABI against the sets of iterative edges the
-unmodified reference wrote (tests/golden_iter/, chain fixtures), against the oracle, through the CLI, and against the
-reference binary itself at 300 k reads with contigs the reference assembled on the GPU box."""
+unmodified reference wrote (tests/golden_iter/, chain fixtures), against the oracle, through the CLI, and against what the
+reference binary wrote at 300 k reads from contigs it assembled (tests/golden/scale/, oracle/scale_golden.py)."""
 import os
 import subprocess
-import time
 
 import numpy as np
 import pytest
 
 from conftest import ROOT
 from megahit_b200 import formats as F
-from megahit_b200 import lib, synth
+from megahit_b200 import lib
 from oracle import oracle as O
+from oracle import scale_golden as SG
 from test_oracle_iter import contig_seqs, iter_cases, iter_inputs
 
 pytestmark = pytest.mark.gpu
 
-REF = os.path.join(ROOT, "oracle", "_ref", "megahit_core_ref")
 OURS = os.path.join(ROOT, "megahit_b200", "bin", "megahit_core")
 
 
@@ -41,15 +40,7 @@ def _run(cmd, **kw):
     return r
 
 
-def _edge_set(prefix):
-    info = open(prefix + ".edges.info").read().split()
-    assert info[0] == "kmer_size" and info[10] == "is_sorted" and info[11] == "0" and info[7] == "0"
-    W, n = int(info[3]), int(info[9])
-    e = np.fromfile(prefix + ".edges.0", np.uint32).reshape(-1, W)
-    assert len(e) == n
-    u = np.unique(e, axis=0)
-    assert len(u) == n
-    return int(info[1]), u
+_edge_set = SG.edge_set
 
 
 def test_cli_iterate_on_fixture(tmp_path):
@@ -63,45 +54,17 @@ def test_cli_iterate_on_fixture(tmp_path):
 
 
 def test_cli_iterate_matches_reference_binary_at_300k_reads(tmp_path):
-    """k = 21 contigs assembled by the reference on the box from a repeat-rich synthetic genome, then `iterate` 21 -> 29 and
-    21 -> 41 by both binaries: same set of edges"""
-    if not os.path.exists(REF):
-        pytest.fail("oracle/_ref/megahit_core_ref is missing")
-    rng = np.random.default_rng(11)
-    n_reads, L, G = 300_000, 150, 1_500_000
-    g = rng.integers(0, 4, G, dtype=np.uint8)
-    for rl, copies in ((30, 400), (45, 300), (70, 200)):
-        rep = rng.integers(0, 4, rl, dtype=np.uint8)
-        for p in rng.choice(G - rl, copies, replace=False):
-            g[p:p + rl] = rep
-    pos = rng.integers(0, G - L + 1, size=n_reads)
-    b = g[pos[:, None] + np.arange(L)[None, :]]
-    rc = rng.integers(0, 2, size=n_reads).astype(bool)
-    b[rc] = 3 - b[rc][:, ::-1]
-    e = rng.random(b.shape) < 0.01
-    b[e] = (b[e] + rng.integers(1, 4, size=int(e.sum()), dtype=np.uint8)) & 3
+    """k = 21 contigs the reference assembled from a repeat-rich synthetic genome, then `iterate` 21 -> 29 and 21 -> 41:
+    the same set of edges as the reference binary wrote"""
     libp = str(tmp_path / "reads.lib")
-    F.write_lib(libp, F.pack_reads_fixed(b), n_reads, n_reads * L, L)
-    t = str(min(32, os.cpu_count() or 8))
-    p21 = str(tmp_path / "k21")
-    _run([REF, "count", "-k", "21", "-m", "2", "--host_mem", "3e10", "--mem_flag", "1", "--output_prefix", p21,
-          "--num_cpu_threads", t, "--read_lib_file", libp])
-    _run([REF, "seq2sdbg", "--host_mem", "3e10", "--mem_flag", "1", "--output_prefix", p21, "--num_cpu_threads", t, "-k", "21",
-          "--kmer_from", "0", "--input_prefix", p21, "--need_mercy"])
-    _run([REF, "assemble", "-s", p21, "-o", p21, "-t", t, "--min_standalone", "200", "--prune_level", "2",
-          "--merge_len", "20", "--merge_similar", "0.95", "--cleaning_rounds", "5", "--disconnect_ratio", "0.1",
-          "--low_local_ratio", "0.2", "--min_depth", "2", "--bubble_level", "2", "--max_tip_len", "-1",
-          "--careful_bubble"], cwd=str(tmp_path))
-    contigs, bubble = p21 + ".contigs.fa", p21 + ".bubble_seq.fa"
-    assert os.path.getsize(contigs) > 0
+    contigs, bubble = SG.write_iter_inputs(str(tmp_path), SG.repeat_genome_and_lib(libp))
+    gold = SG.golden()["iterate_300k"]["steps"]
     for step in (8, 20):
-        res = {}
-        for name, core in (("ref", REF), ("ours", OURS)):
-            p = str(tmp_path / f"{name}_{step}")
-            t0 = time.time()
-            r = _run([core, "iterate", "-c", contigs, "-b", bubble, "-t", t, "-k", "21", "-s", str(step), "-o", p, "-r", libp + ".bin"])
-            res[name] = _edge_set(p)
-            gpu = [l for l in r.stderr.splitlines() if "iterate done" in l]
-            print(f"iterate 21+{step} {name}: {time.time() - t0:.2f} s wall, {len(res[name][1])} edges {gpu[-1].split('- ')[-1] if gpu else ''}")
-        assert res["ours"][0] == res["ref"][0] == 21 + step
-        assert len(res["ref"][1]) > 100 and (res["ours"][1] == res["ref"][1]).all()
+        p = str(tmp_path / f"ours_{step}")
+        r = _run(SG.iterate_argv(OURS, contigs, bubble, libp, p, step, min(32, os.cpu_count() or 8)))
+        ks, u = _edge_set(p)
+        gpu = [l for l in r.stderr.splitlines() if "iterate done" in l]
+        print(f"iterate 21+{step}: {len(u)} edges {gpu[-1].split('- ')[-1] if gpu else ''}")
+        want = gold[str(step)]
+        assert ks == want["kmer_size"] == 21 + step
+        assert len(u) == want["n_edges"] > 100 and F.sha256(u.tobytes()) == want["edges_sha256"]

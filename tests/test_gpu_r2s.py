@@ -7,23 +7,25 @@
   far above kmsort's insertion-sort threshold, where the reference's result depends on kmsort's order among tied
   records (a stable sort gives other bytes - checked on the oracle, tests/test_oracle_r2s.py);
 * the oracle on the intermediate state (solid-edge bits are not visible through the ABI; the SdBG is);
-* the reference binary itself on the GPU box at 300 k reads, through the CLI (`megahit_core read2sdbg`).
+* the reference binary's output at 300 k reads (digests in tests/golden/scale/), through the CLI (`megahit_core read2sdbg`).
 """
+import json
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 from conftest import ROOT
 from megahit_b200 import formats as F
-from megahit_b200 import lib, synth
+from megahit_b200 import lib
 from oracle import oracle as O
+from oracle import scale_golden as SG
 from test_oracle_r2s import R2S, r2s_reads
 
 pytestmark = pytest.mark.gpu
 
-REF = os.path.join(ROOT, "oracle", "_ref", "megahit_core_ref")
 OURS = os.path.join(ROOT, "megahit_b200", "bin", "megahit_core")
 
 
@@ -92,43 +94,33 @@ def _run(cmd, **kw):
     return r
 
 
-def _sdbg_digest(p):
-    info, stream, table = F.canonical_sdbg(p)
-    return {"sdbg": F.sha256(stream), "k": info.k, "wpt": info.words_per_tip_label, "items": int(table[:, 0].sum()),
-            "tips": int(table[:, 1].sum()), "large": int(table[:, 2].sum())}
-
-
 @pytest.mark.parametrize("m,mercy", [(2, True), (1, False)])
 def test_cli_read2sdbg_matches_reference_binary_at_300k_reads(tmp_path, m, mercy):
-    """the sub-command itself, against the reference binary run on the same box; buckets of ~600 stage-1 records
-    (kmsort's radix levels decide the tie order), 37 M stage-1 records, 70+ M stage-2 items"""
-    if not os.path.exists(REF):
-        pytest.fail("oracle/_ref/megahit_core_ref is missing (built in the container, travels with the snapshot)")
-    n_reads, L = 300_000, 150
-    b = synth.synth_reads(n_reads, L, 5 * n_reads, 0.01, seed=777)
+    """the sub-command itself, against what the reference binary wrote for the same seeded library; buckets of ~600
+    stage-1 records (kmsort's radix levels decide the tie order), 37 M stage-1 records, 70+ M stage-2 items"""
     libp = str(tmp_path / "reads.lib")
-    F.write_lib(libp, b, n_reads, n_reads * L, L)
-    res = {}
-    for name, core in (("ref", REF), ("ours", OURS)):
-        p = str(tmp_path / name)
-        cmd = [core, "read2sdbg", "-k", "27", "-m", str(m), "--host_mem", "3e10", "--mem_flag", "1", "--output_prefix", p,
-               "--num_cpu_threads", str(min(32, os.cpu_count() or 8)), "--read_lib_file", libp]
-        _run(cmd + (["--need_mercy"] if mercy else []))
-        res[name] = _sdbg_digest(p)
-        if m > 1:
-            res[name]["counting"] = F.file_sha256(p + ".counting")
-        assert os.path.exists(p + ".mercy_cand.0")
-    assert res["ours"] == res["ref"]
+    SG.r2s_lib(libp)
+    p = str(tmp_path / "ours")
+    _run(SG.r2s_argv(OURS, libp, p, m, mercy, min(32, os.cpu_count() or 8)))
+    got = SG.sdbg_digests(p)
+    if m > 1:
+        got["counting"] = F.file_sha256(p + ".counting")
+    assert os.path.exists(p + ".mercy_cand.0")
+    assert got == SG.golden()["read2sdbg_300k_k27"][f"m{m}_mercy{int(mercy)}"]
 
 
 def test_cli_forwards_wide_stage1_to_reference(tmp_path):
-    """k = 255 with min count 2: stage-1 records of 19 words are outside the device sort; the CLI hands the command to
-    the reference binary (MHB_REFERENCE_CORE) instead of failing"""
-    if not os.path.exists(REF):
-        pytest.fail("oracle/_ref/megahit_core_ref is missing")
+    """k = 255 with min count 2: stage-1 records of 19 words are outside the device sort; the CLI hands the command,
+    unchanged, to the reference binary (MHB_REFERENCE_CORE) instead of failing.  tests/ref_stand_in.py stands in for
+    the reference: it records its command line and writes the SdBG the reference writes for this library."""
     gold = [r for r in R2S["runs"] if r["k"] == 255 and r["m"] == 2][0]
     p = str(tmp_path / "o")
-    env = dict(os.environ, MHB_REFERENCE_CORE=REF)
-    _run([OURS, "read2sdbg", "-k", "255", "-m", "2", "--host_mem", "3e10", "--output_prefix", p, "--num_cpu_threads", "4",
-          "--read_lib_file", os.path.join(ROOT, "tests", gold["lib"], "reads.lib"), "--need_mercy"], env=env)
-    assert _sdbg_digest(p)["sdbg"] == gold["sdbg_sha256"]
+    stand_in = tmp_path / "megahit_core_ref"
+    stand_in.write_text(f"#!{sys.executable}\nimport sys\nsys.path.insert(0, {os.path.join(ROOT, 'tests')!r})\n"
+                        "import ref_stand_in\nref_stand_in.main(sys.argv)\n")
+    stand_in.chmod(0o755)
+    args = ["read2sdbg", "-k", "255", "-m", "2", "--host_mem", "3e10", "--output_prefix", p, "--num_cpu_threads", "4",
+            "--read_lib_file", os.path.join(ROOT, "tests", gold["lib"], "reads.lib"), "--need_mercy"]
+    _run([OURS] + args, env=dict(os.environ, MHB_REFERENCE_CORE=str(stand_in)))
+    assert json.load(open(p + ".argv.json")) == [str(stand_in)] + args
+    assert F.sha256(F.canonical_sdbg(p)[1]) == gold["sdbg_sha256"]
