@@ -6,8 +6,8 @@
 //   1. three stable radix passes on the three leading key bytes (the same k_radix_pass3 the sort uses) group the
 //      records by their leading 24 key bits - 3 x 2NS bytes instead of 7 x 2NS;
 //   2. k_bucket_bounds finds the 65 537 boundaries of the reference's 16-bit buckets (base_engine.h kNumBuckets) by
-//      binary search, and every bucket is cut into slices of ~6000 records whose boundaries are moved to the next
-//      change of the 24-bit prefix: a slice is contiguous and key-closed;
+//      binary search, and k_slice_table cuts every bucket into slices of ~6000 records whose boundaries are moved to
+//      the next change of the 24-bit prefix: a slice is contiguous and key-closed;
 //   3. k_hash_count: a CTA takes a slice and aggregates it in a shared-memory open-addressing table keyed by the
 //      remaining 42 record bits: occurrence counts first, then, for the keys that reached the solid threshold, the
 //      4 + 4 prev/next tallies (has_in / has_out, :279-305) in a second sweep over the same records (L2 hits); the solid
@@ -167,39 +167,64 @@ __device__ __forceinline__ bool hc_any_byte_ge(u32 w, u32 m) {
   return (w & 0xFFu) >= m || ((w >> 8) & 0xFFu) >= m || ((w >> 16) & 0xFFu) >= m || (w >> 24) >= m;
 }
 
-// first index q in [p, hi] that may start a slice: q == lo, q == hi, or the 24-bit prefix changes between q-1 and q
-// (records with equal keys share their prefix, so they never straddle such a boundary).  Block-wide.
-template <int THREADS>
-__device__ __forceinline__ u64 hc_align(const uint2 *__restrict__ recs, u64 p, u64 lo, u64 hi, u32 *s_min) {
-  if (p <= lo) return lo;
-  if (p >= hi) return hi;
-  for (u64 q0 = p; q0 < hi; q0 += THREADS) {
-    __syncthreads();
-    if (threadIdx.x == 0) *s_min = 0xFFFFFFFFu;
-    __syncthreads();
-    const u64 q = q0 + threadIdx.x;
-    if (q < hi && (recs[q].x >> 8) != (recs[q - 1].x >> 8)) atomicMin(s_min, threadIdx.x);
-    __syncthreads();
-    const u32 f = *s_min;
-    if (f != 0xFFFFFFFFu) return q0 + f;
+// Slice table: bucket b (16-bit prefix) is cut into ceil(n_b / T) slices whose boundaries are moved forward to the next
+// change of the 24-bit prefix, so that a slice is a contiguous, key-closed range (records with equal keys share their
+// prefix, so they never straddle such a boundary).  slice_off[b] = first slice id of bucket b (exclusive scan of the
+// per-bucket slice counts).  One thread per slice: slice_start[s] = first record of slice s, slice_start[n_slices] = n
+// (the end of a slice is the start of the next one), slice_bucket[s] = its bucket, slice_base[s] = where its solid
+// entries go in the scratch list: list[a_s / m + s ...) with a_s the slice's first record (a slice of n records holds at
+// most n / m solid keys and floor is super-additive: the areas never overlap).  Computed up front so that a hash CTA
+// starts a slice with two loads instead of a serial search and block-wide boundary scans.
+__global__ void k_slice_table(const uint2 *__restrict__ recs, const u64 *__restrict__ bounds, const u64 *__restrict__ slice_off,
+                              const u64 *__restrict__ n_slices_dev, u64 n, int m, u64 *__restrict__ slice_start,
+                              u64 *__restrict__ slice_base, u32 *__restrict__ slice_bucket) {
+  const u64 sl = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  const u64 n_slices = *n_slices_dev;
+  if (sl > n_slices) return;
+  if (sl == n_slices) {
+    slice_start[sl] = n;
+    return;
   }
-  return hi;
+  u32 a = 0, z = 65536;  // bucket of this slice: last b with slice_off[b] <= sl
+  while (z - a > 1) {
+    const u32 mid = (a + z) >> 1;
+    if (slice_off[mid] <= sl) a = mid;
+    else z = mid;
+  }
+  const u32 b = a;
+  const u64 blo = bounds[b], bhi = bounds[b + 1];
+  const u64 n_in_b = slice_off[b + 1] - slice_off[b], idx = sl - slice_off[b];
+  const u64 step = (bhi - blo + n_in_b - 1) / n_in_b;
+  const u64 p = blo + idx * step;
+  u64 lo;
+  if (p <= blo) {
+    lo = blo;
+  } else if (p >= bhi) {
+    lo = bhi;
+  } else {  // first q in [p, bhi) whose 24-bit prefix exceeds that of record p - 1 (sorted on it), else bhi
+    const u32 g = recs[p - 1].x >> 8;
+    u64 l = p, h = bhi;
+    while (l < h) {
+      const u64 mid = (l + h) >> 1;
+      if ((recs[mid].x >> 8) <= g) l = mid + 1;
+      else h = mid;
+    }
+    lo = l;
+  }
+  slice_start[sl] = lo;
+  slice_base[sl] = lo / (u64)m + sl;
+  slice_bucket[sl] = b;
 }
 
-// Work unit = a SLICE of the prefix-sorted records: bucket b (16-bit prefix) is cut into ceil(n_b / T) slices whose
-// boundaries are moved forward to the next change of the 24-bit prefix, so that a slice is a contiguous, key-closed
-// range read once with every lane busy.  slice_off[b] = first slice id of bucket b (exclusive scan of the per-bucket
-// slice counts).  list: slice s's solid entries go to list[a_s / m + s ...) with a_s the slice's first record (a slice
-// of n records holds at most n / m solid keys and floor is super-additive: the areas never overlap).
+// Work unit = a slice of the slice table, taken by ticket (the next ticket is requested a whole slice ahead), read
+// once with every lane busy.
 // One sweep per slice: occurrence count and the 4 + 4 prev / next tallies (kmer_counter.cpp:279-295) of every key, the
 // tallies as byte fields; only keys with >= 256 occurrences ("hot": a byte could wrap) get a second sweep with exact
 // 32-bit tallies, 32 keys at a time.
 template <class G>
 __global__ void __launch_bounds__(G::THREADS, G::CTAS)
-    k_hash_count(const uint2 *__restrict__ recs, const u64 *__restrict__ bounds, const u64 *__restrict__ slice_off,
-                 const u64 *__restrict__ n_slices_dev, int m, u32 *ticket, u64 *__restrict__ list,
-                 u32 *__restrict__ slice_count, u64 *__restrict__ slice_base, u32 *__restrict__ slice_bucket, u64 *mul_hist,
-                 u32 *err_flag) {
+    k_hash_count(const uint2 *__restrict__ recs, const u64 *__restrict__ slice_start, const u64 *__restrict__ n_slices_dev,
+                 int m, u32 *ticket, u64 *__restrict__ list, u32 *__restrict__ slice_count, u64 *mul_hist, u32 *err_flag) {
   constexpr int THREADS = G::THREADS, SLOTS = G::SLOTS, MAX_SOLID = G::MAX_SOLID, CELLS = G::CELLS;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   HcShared<G> &s = *reinterpret_cast<HcShared<G> *>(smem_raw);
@@ -214,34 +239,18 @@ __global__ void __launch_bounds__(G::THREADS, G::CTAS)
   __syncthreads();
   const u64 n_slices = *n_slices_dev;
   const u32 um = (u32)m;
+  u32 next = tid == 0 ? atomicAdd(ticket, 1u) : 0u;
   while (true) {
     if (tid == 0) {
-      const u32 sl = atomicAdd(ticket, 1u);
-      s.bucket = sl;
-      if (sl < n_slices) {  // bucket of this slice: last b with slice_off[b] <= sl
-        u32 a = 0, z = 65536;
-        while (z - a > 1) {
-          const u32 mid = (a + z) >> 1;
-          if (slice_off[mid] <= sl) a = mid; else z = mid;
-        }
-        s.sp = a;
-      }
+      s.bucket = next;
+      next = atomicAdd(ticket, 1u);  // tickets only grow: once this one is past the end, so is the prefetched one
     }
     __syncthreads();
     const u32 sl = s.bucket;
     if (sl >= n_slices) break;
-    const u32 b = s.sp;
-    __syncthreads();
-    const u64 blo = bounds[b], bhi = bounds[b + 1];
-    const u64 n_in_b = slice_off[b + 1] - slice_off[b], idx = sl - slice_off[b];
-    const u64 step = (bhi - blo + n_in_b - 1) / n_in_b;
-    const u64 lo = hc_align<THREADS>(recs, blo + idx * step, blo, bhi, &s.overflow);
-    const u64 hi = idx + 1 == n_in_b ? bhi : hc_align<THREADS>(recs, blo + (idx + 1) * step, blo, bhi, &s.overflow);
-    __syncthreads();
+    const u64 lo = slice_start[sl], hi = slice_start[sl + 1];
     const u64 base = lo / (u64)m + sl;
     if (tid == 0) {
-      slice_base[sl] = base;
-      slice_bucket[sl] = b;
       s.out_cursor = 0;
       s.st_prefix[0] = 0;
       s.st_bits[0] = 0;
@@ -499,8 +508,8 @@ static u32 hc_slice_records() {
 #define kHcSliceRecords hc_slice_records()
 
 template <class G>
-static int launch_hash_count(cudaStream_t st, const uint2 *recs, const u64 *bounds, const u64 *slice_off, const u64 *n_slices_dev,
-                             int m, u32 *misc, u64 *list, u32 *slice_count, u64 *slice_base, u32 *slice_bucket, u64 *mul_hist) {
+static int launch_hash_count(cudaStream_t st, const uint2 *recs, const u64 *slice_start, const u64 *n_slices_dev, int m,
+                             u32 *misc, u64 *list, u32 *slice_count, u64 *mul_hist) {
   static int bps = 0;
   const size_t smem = sizeof(HcShared<G>);
   if (!bps) {
@@ -509,14 +518,15 @@ static int launch_hash_count(cudaStream_t st, const uint2 *recs, const u64 *boun
     if (bps < 1) return mhb_set_error(MHB_ERR_CUDA, "hash-count kernel does not fit an SM (%zu B shared memory)", smem);
     if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] hash count: %d threads, %d slots, %zu B smem, %d CTA/SM, slice %u\n", G::THREADS, G::SLOTS, smem, bps, kHcSliceRecords);
   }
-  k_hash_count<G><<<sm_count() * bps, G::THREADS, smem, st>>>(recs, bounds, slice_off, n_slices_dev, m, misc, list, slice_count,
-                                                             slice_base, slice_bucket, mul_hist, misc + 1);
+  k_hash_count<G><<<sm_count() * bps, G::THREADS, smem, st>>>(recs, slice_start, n_slices_dev, m, misc, list, slice_count,
+                                                             mul_hist, misc + 1);
   CK_LAUNCH();
   return MHB_OK;
 }
 
 struct HcLayout {
-  size_t sort_ws, off_bounds, off_bcnt, off_soff, off_bsum, off_misc, off_scount, off_sdst, off_sbase, off_sbucket, off_list, total;
+  size_t sort_ws, off_bounds, off_bcnt, off_soff, off_bsum, off_misc, off_scount, off_sdst, off_sbase, off_sbucket, off_sstart,
+      off_list, total;
   uint64_t max_slices;
 };
 HcLayout hc_layout(uint64_t n, int32_t m) {
@@ -543,6 +553,8 @@ HcLayout hc_layout(uint64_t n, int32_t m) {
   p += pad(L.max_slices * 8);
   L.off_sbucket = p;
   p += pad(L.max_slices * 4);
+  L.off_sstart = p;
+  p += pad((L.max_slices + 1) * 8);
   L.off_list = p;
   p += pad((size_t)(n / (uint64_t)(m < 1 ? 1 : m) + L.max_slices + 8) * 8);
   L.total = p;
@@ -586,6 +598,7 @@ extern "C" int mhb_count_solid_hashed(void *stream, uint32_t *recs_a, uint32_t *
   u64 *slice_dst = (u64 *)(w + L.off_sdst);
   u64 *slice_base = (u64 *)(w + L.off_sbase);
   u32 *slice_bucket = (u32 *)(w + L.off_sbucket);
+  u64 *slice_start = (u64 *)(w + L.off_sstart);
   u64 *list = (u64 *)(w + L.off_list);
   u64 *n_slices_dev = (u64 *)(misc + 2);
   CK(cudaMemsetAsync(misc, 0, 256, st));
@@ -597,12 +610,15 @@ extern "C" int mhb_count_solid_hashed(void *stream, uint32_t *recs_a, uint32_t *
   CK_LAUNCH();
   if (int rc = scan_counts(st, bcnt, 65536, slice_off, n_slices_dev, bsum)) return rc;
   CK(cudaMemcpyAsync(slice_off + 65536, n_slices_dev, 8, cudaMemcpyDeviceToDevice, st));
+  k_slice_table<<<(unsigned)((L.max_slices + 1 + 255) / 256), 256, 0, st>>>(recs, bounds, slice_off, n_slices_dev, n, m, slice_start,
+                                                                            slice_base, slice_bucket);
+  CK_LAUNCH();
   // 3. per-slice hash aggregation
   {
     int rc;
-    if (hc_geom() == 0) rc = launch_hash_count<HcGeomA>(st, recs, bounds, slice_off, n_slices_dev, m, misc, list, slice_count, slice_base, slice_bucket, mul_hist);
-    else if (hc_geom() == 2) rc = launch_hash_count<HcGeomC>(st, recs, bounds, slice_off, n_slices_dev, m, misc, list, slice_count, slice_base, slice_bucket, mul_hist);
-    else rc = launch_hash_count<HcGeomB>(st, recs, bounds, slice_off, n_slices_dev, m, misc, list, slice_count, slice_base, slice_bucket, mul_hist);
+    if (hc_geom() == 0) rc = launch_hash_count<HcGeomA>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
+    else if (hc_geom() == 2) rc = launch_hash_count<HcGeomC>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
+    else rc = launch_hash_count<HcGeomB>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
     if (rc) return rc;
   }
   // 4. offsets + edges (the scan runs over the allocated maximum; unused slice ids hold zero)
