@@ -122,17 +122,17 @@ int mhb_sort_records(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint32_
 int mhb_sort_records_relaxed(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint32_t words, const uint8_t *bytes,
                              uint32_t n_bytes, const uint64_t *first_hist, void *ws, size_t ws_bytes, int *result_in_b);
 
-/* Fused partition + exchange for the multi-GPU path: ONE stable radix pass whose per-digit destinations are arbitrary
+/* Fused partition + exchange for the multi-GPU path: ONE unstable radix pass whose per-digit destinations are arbitrary
  * device byte addresses (bin_addr_dev[256], device memory) = where the first record of digit d coming from THIS call
  * goes.  The digit of a record is owner_of_byte_dev[record byte `byte`] (256-entry device table mapping the record's
- * leading byte to the owning rank) or the byte itself when that table is NULL.  Digits owned by another GPU point
- * into that GPU's receive buffer (opened with mhb_ipc_open), so the scatter stores cross NVLink inside the sorting
- * kernel and no separate all-to-all is needed.  ws as for mhb_sort_records. */
+ * leading byte to the owning rank; required).  Digits owned by another GPU point into that GPU's receive buffer (opened
+ * with mhb_ipc_open), so the scatter stores cross NVLink inside the partitioning kernel and no separate all-to-all is
+ * needed.  The order of the records inside an owner's block is unspecified.  ws as for mhb_sort_records. */
 int mhb_partition_scatter(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
                           const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws, size_t ws_bytes);
-/* The same pass, additionally delivering - where the pass variant supports it (*hist_done = 1; 8- and 12-byte records) -
- * one histogram of record byte `next_byte` per owner: owner_next_hist[o * 256 + v] (device uint64[16 * 256],
- * caller-zeroed) += records sent to owner o whose byte next_byte is v.  Summed over the sending ranks it is the
+/* The same pass, additionally delivering one histogram of record byte `next_byte` per owner (*hist_done = 1 on
+ * success): owner_next_hist[o * 256 + v] (device uint64[16 * 256], caller-zeroed) += records sent to owner o whose byte
+ * next_byte is v.  Summed over the sending ranks it is the
  * first-pass histogram of the owner's sort, which then need not sweep its records to count. */
 int mhb_partition_scatter_hist(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
                                const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws, size_t ws_bytes,
@@ -158,10 +158,6 @@ int mhb_dev_free(void *ptr);
 int mhb_ipc_export(const void *dev_ptr, uint8_t *handle64);
 int mhb_ipc_open(const uint8_t *handle64, void **peer_ptr);
 int mhb_ipc_close(void *peer_ptr);
-
-/* Tuning hook: selects the tile geometry / ranking variant of the radix pass for subsequent sorts (0 = default;
- * also read once from the environment variable MHB_SORT_CFG).  Every variant produces the same output. */
-int mhb_set_sort_cfg(int cfg);
 
 /* Per-pass device times (ms, CUDA events on `stream`) of one of the last four sorts issued by this process:
  * back = 0 is the most recent.  Synchronises on that sort's last event only. */

@@ -115,46 +115,6 @@ __global__ void __launch_bounds__(kExtractThreads)
 }
 
 // ------------------------------------------------------------------------------------------------
-// K-extract, rolling variant for 8-byte records (17 <= k+1 <= 29; opt-in: MHB_EXTRACT_ROLL=1): a lane builds FOUR
-// consecutive records, the first from the packed words, the other three by rolling the forward / reverse /
-// complement strings one base on (make_count_records_roll): ~55 instead of ~120 thread-instructions per record.
-// A 150 bp read at k=27 (123 edges) is one warp step.  Same output as k_count_extract<2, 2>.
-// ------------------------------------------------------------------------------------------------
-static __global__ void __launch_bounds__(kExtractThreads)
-    k_count_extract_roll(ReadsView rv, u32 k, u32 *__restrict__ records, u64 *hist, int hist_byte) {
-  __shared__ u32 s_hist[256];
-  for (int i = threadIdx.x; i < 256; i += kExtractThreads) s_hist[i] = 0;
-  const u32 lane = lane_id();
-  const u32 K1 = k + 1;
-  const u32 hshift = 8u * (u32)hist_byte;
-  for_each_read(rv, [&](u64 r, const u32 *s, u32 nwords, u32 L) {
-    if (L < K1) return;  // kmer_counter.cpp:124
-    const u32 n_e = L - k;
-    const u64 base = rv.fixed_len ? r * (u64)(rv.fixed_len - k) : rv.edge_off[r];
-    for (u32 q0 = 0; q0 < n_e; q0 += 128) {
-      const u32 q = q0 + 4 * lane;
-      if (q < n_e) {
-        u64 rec[4];
-        u32 strand[4];
-        make_count_records_roll<4>(s, nwords, L, k, q, rec, strand);
-        const u32 cnt = n_e - q < 4u ? n_e - q : 4u;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if ((u32)j < cnt) {
-            reinterpret_cast<uint2 *>(records)[base + q + j] = make_uint2((u32)(rec[j] >> 32), (u32)rec[j]);
-            if (hist) atomicAdd(&s_hist[(u32)(rec[j] >> hshift) & 255u], 1u);
-          }
-        }
-      }
-    }
-  });
-  __syncthreads();
-  if (hist)
-    for (int i = threadIdx.x; i < 256; i += kExtractThreads)
-      if (s_hist[i]) atomicAdd((unsigned long long *)&hist[i], (unsigned long long)s_hist[i]);
-}
-
-// ------------------------------------------------------------------------------------------------
 // K-extract restricted to a range of leading bytes (A13; base_engine.cpp:254-281 Lv1 passes over bucket ranges):
 // when the records of a whole library do not fit in HBM the count stage runs in rounds, each round extracting only
 // the edges whose first eight bases (the 16-bit bucket id) lie in [lo, hi].  Two launches, no atomics, read order kept:
@@ -408,8 +368,8 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-// Rolling variant of k_mark_mercy for 8-byte records (opt-in with MHB_EXTRACT_ROLL=1): a lane re-derives four
-// consecutive canonical (k+1)-mers with make_count_records_roll and probes the filter for all four at once.
+// Rolling variant of k_mark_mercy for 8-byte records: a lane re-derives four consecutive canonical (k+1)-mers with
+// make_count_records_roll (~55 instead of ~120 thread-instructions per record) and probes the filter for all four at once.
 static __global__ void __launch_bounds__(256)
     k_mark_mercy_roll(ReadsView rv, u32 k, const u32 *__restrict__ filter, u64 filter_words, const u32 *__restrict__ table,
                       u64 cap, u32 *first_0_out, u32 *last_0_in) {

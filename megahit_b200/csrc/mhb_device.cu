@@ -157,12 +157,6 @@ extern "C" int mhb_count_extract(void *stream, const mhb_dev_reads *reads, uint3
   const u32 W = count_key_words(k), WR = count_record_words(k);
   const u64 n_batches = (rv.n_reads + kReadsPerBatch - 1) / kReadsPerBatch;
   const int grid = (int)(n_batches < (u64)(sm_count() * 8) ? n_batches : (u64)(sm_count() * 8));
-  static const bool roll = getenv("MHB_EXTRACT_ROLL") && !strcmp(getenv("MHB_EXTRACT_ROLL"), "1");  // opt-in (no gain measured)
-  if (roll && W == 2 && WR == 2 && k + 1 >= 17) {
-    k_count_extract_roll<<<grid, kExtractThreads, 0, st>>>(rv, k, records, hist256, hist_byte);
-    CK_LAUNCH();
-    return MHB_OK;
-  }
 #define M(WW)                                                                                              \
   if (W == WW && WR == WW)                                                                                 \
     k_count_extract<WW, WW><<<grid, kExtractThreads, 0, st>>>(rv, k, records, hist256, hist_byte);         \
@@ -338,6 +332,15 @@ extern "C" int mhb_tipset_build(void *stream, const uint32_t *edges, const uint8
   return MHB_OK;
 }
 
+// 8-byte records (W == 2 implies k + 1 >= 17) take the rolling record builder, 4 positions per lane, three of them by
+// shifting: 6.5 vs 7.4 ms for the per-position kernel on the bench workload (profiles/r2a_bench_roll.json)
+template <int W, int WR>
+static void launch_mark_mercy(cudaStream_t st, int grid, const ReadsView &rv, u32 k, const u32 *filter, u64 fwords,
+                              const u32 *table, u64 cap, u32 *first_0_out, u32 *last_0_in) {
+  if constexpr (W == 2 && WR == 2) k_mark_mercy_roll<<<grid, 256, 0, st>>>(rv, k, filter, fwords, table, cap, first_0_out, last_0_in);
+  else k_mark_mercy<W, WR><<<grid, 256, 0, st>>>(rv, k, filter, fwords, table, cap, first_0_out, last_0_in);
+}
+
 extern "C" int mhb_count_mark_mercy(void *stream, const mhb_dev_reads *reads, uint32_t k, const void *tipset,
                                     size_t tipset_bytes, uint64_t n_tip_edges, uint32_t *first_0_out,
                                     uint32_t *last_0_in) {
@@ -353,19 +356,11 @@ extern "C" int mhb_count_mark_mercy(void *stream, const mhb_dev_reads *reads, ui
   u64 g64 = (rv.n_reads + 7) / 8;
   if (g64 > (u64)sm_count() * 16) g64 = (u64)sm_count() * 16;
   const int grid = (int)g64;
-  // rolling record builder (4 positions per lane, three of them by shifting): 6.5 vs 7.4 ms on the bench workload
-  // (profiles/r2a_bench_roll.json); MHB_EXTRACT_ROLL=0 selects the per-position kernel
-  static const bool roll = !(getenv("MHB_EXTRACT_ROLL") && !strcmp(getenv("MHB_EXTRACT_ROLL"), "0"));
-  if (roll && W == 2 && WR == 2 && k + 1 >= 17) {
-    k_mark_mercy_roll<<<grid, 256, 0, st>>>(rv, k, filter, fwords, table, cap, first_0_out, last_0_in);
-    CK_LAUNCH();
-    return MHB_OK;
-  }
 #define M(WW)                                                                                                          \
   if (W == WW && WR == WW)                                                                                             \
-    k_mark_mercy<WW, WW><<<grid, 256, 0, st>>>(rv, k, filter, fwords, table, cap, first_0_out, last_0_in);              \
+    launch_mark_mercy<WW, WW>(st, grid, rv, k, filter, fwords, table, cap, first_0_out, last_0_in);                    \
   else if (W == WW && WR == WW + 1)                                                                                    \
-    k_mark_mercy<WW, WW + 1><<<grid, 256, 0, st>>>(rv, k, filter, fwords, table, cap, first_0_out, last_0_in);          \
+    launch_mark_mercy<WW, WW + 1>(st, grid, rv, k, filter, fwords, table, cap, first_0_out, last_0_in);                \
   else
   MHB_FOR_W(M) return mhb_set_error(MHB_ERR_ARG, "unsupported k=%u", k);
 #undef M
@@ -504,11 +499,8 @@ static u32 emit2_chunk_records(u32 W) {
 extern "C" size_t mhb_s2s_emit_scratch_bytes(uint64_t n, uint32_t k) {
   const u32 W = s2s_record_words(k);
   const u64 nc = emit2_chunks(n, W);
-  const u64 nblk = (n + kEmitThreads - 1) / kEmitThreads;  // v1 layout (MHB_EMIT_V1)
-  const size_t v1 = (size_t)nblk * 4 * 8 + (size_t)MHB_NUM_BUCKETS * 4 * 8 + (size_t)(nblk / kScanTile + 2) * 8 + 512;
-  const size_t v2 = (size_t)MHB_NUM_BUCKETS * (4 * 8 + 5 * 4) + (size_t)nc * 4 * (4 + 8) + (size_t)(nc / kScanTile + 2) * 8 +
-                    (size_t)nc * emit2_chunk_records(W) * emit2_max_item_bytes(k) + 4096;
-  return v1 > v2 ? v1 : v2;
+  return (size_t)MHB_NUM_BUCKETS * (4 * 8 + 5 * 4) + (size_t)nc * 4 * (4 + 8) + (size_t)(nc / kScanTile + 2) * 8 +
+         (size_t)nc * emit2_chunk_records(W) * emit2_max_item_bytes(k) + 4096;
 }
 
 extern "C" int mhb_s2s_emit(void *stream, const uint32_t *sorted_records, uint64_t n, uint32_t k, uint8_t *bytes_out,
@@ -529,24 +521,22 @@ extern "C" int mhb_s2s_emit_fmt(void *stream, const uint32_t *sorted_records, ui
   if (n == 0) return MHB_OK;
   if (scratch_bytes < mhb_s2s_emit_scratch_bytes(n, k)) return mhb_set_error(MHB_ERR_ARG, "emit scratch too small");
   const u32 W = s2s_record_words(k);
-  static const bool use_v1 = getenv("MHB_EMIT_V1") != nullptr;
-  if (!use_v1) {
-    const u64 nc = emit2_chunks(n, W);
-    if (nc >= (1ull << 32)) return mhb_set_error(MHB_ERR_ARG, "too many records for one emit launch");
-    const u32 chrec = emit2_chunk_records(W), maxb = emit2_max_item_bytes(k);
-    char *p = (char *)scratch;
-    u64 *bucket_start = (u64 *)p;
-    p += (size_t)MHB_NUM_BUCKETS * 4 * 8;
-    u32 *bucket_local = (u32 *)p;
-    p += (size_t)MHB_NUM_BUCKETS * 5 * 4;
-    u64 *chunk_off = (u64 *)p;
-    p += (size_t)nc * 4 * 8;
-    u64 *bsum = (u64 *)p;
-    p += (size_t)(nc / kScanTile + 2) * 8;
-    u32 *chunk_tot = (u32 *)p;
-    p += ((size_t)nc * 4 * 4 + 255) & ~(size_t)255;
-    uint8_t *tmp = (uint8_t *)p;
-    CK(cudaMemsetAsync(bucket_local, 0xFF, (size_t)MHB_NUM_BUCKETS * 5 * 4, st));
+  const u64 nc = emit2_chunks(n, W);
+  if (nc >= (1ull << 32)) return mhb_set_error(MHB_ERR_ARG, "too many records for one emit launch");
+  const u32 chrec = emit2_chunk_records(W), maxb = emit2_max_item_bytes(k);
+  char *p = (char *)scratch;
+  u64 *bucket_start = (u64 *)p;
+  p += (size_t)MHB_NUM_BUCKETS * 4 * 8;
+  u32 *bucket_local = (u32 *)p;
+  p += (size_t)MHB_NUM_BUCKETS * 5 * 4;
+  u64 *chunk_off = (u64 *)p;
+  p += (size_t)nc * 4 * 8;
+  u64 *bsum = (u64 *)p;
+  p += (size_t)(nc / kScanTile + 2) * 8;
+  u32 *chunk_tot = (u32 *)p;
+  p += ((size_t)nc * 4 * 4 + 255) & ~(size_t)255;
+  uint8_t *tmp = (uint8_t *)p;
+  CK(cudaMemsetAsync(bucket_local, 0xFF, (size_t)MHB_NUM_BUCKETS * 5 * 4, st));
 #define M(WW)                                                                                                       \
   if (W == WW) {                                                                                                    \
     const size_t smem = (size_t)kEmit2Warps * emit2_slots(WW) * WW * 4;                                             \
@@ -561,39 +551,16 @@ extern "C" int mhb_s2s_emit_fmt(void *stream, const uint32_t *sorted_records, ui
     k_s2s_judge<WW><<<(unsigned)grid, kEmit2Warps * 32, smem, st>>>(sorted_records, n, k, (u32)nc, tmp, chunk_tot,   \
                                                                    bucket_local, totals, fmt);                     \
   }
-    MHB_FOR_WR(M)
-#undef M
-    CK_LAUNCH();
-    for (int q = 0; q < 4; ++q)
-      if (int rc = scan32(st, chunk_tot + (u64)q * nc, nc, chunk_off + (u64)q * nc, totals + q, bsum)) return rc;
-    u64 gg = (nc + 7) / 8;
-    if (gg > (u64)sm_count() * 16) gg = (u64)sm_count() * 16;
-    k_s2s_gather<<<(unsigned)gg, 256, 0, st>>>(tmp, chrec, maxb, (u32)nc, chunk_tot, chunk_off, bytes_out, capacity_bytes);
-    CK_LAUNCH();
-    k_bucket_starts<<<64, 256, 0, st>>>(bucket_local, chunk_off, nc, bucket_start);
-    CK_LAUNCH();
-    k_bucket_finalize<<<1, 1024, 0, st>>>(bucket_start, totals, bucket_table);
-    CK_LAUNCH();
-    return MHB_OK;
-  }
-  const u64 nblk = (n + kEmitThreads - 1) / kEmitThreads;
-  u64 *bucket_start = (u64 *)scratch;
-  u64 *btot = bucket_start + (size_t)MHB_NUM_BUCKETS * 4;
-  CK(cudaMemsetAsync(bucket_start, 0xFF, (size_t)MHB_NUM_BUCKETS * 4 * 8, st));
-#define M(WW) \
-  if (W == WW) k_s2s_size<WW><<<(unsigned)nblk, kEmitThreads, 0, st>>>(sorted_records, n, k, btot);
   MHB_FOR_WR(M)
 #undef M
   CK_LAUNCH();
-  u64 *bsum = btot + 4 * nblk;
   for (int q = 0; q < 4; ++q)
-    if (int rc = scan64(st, btot + (u64)q * nblk, nblk, totals + q, bsum)) return rc;
-#define M(WW)                                                                                                    \
-  if (W == WW)                                                                                                   \
-    k_s2s_write<WW><<<(unsigned)nblk, kEmitThreads, 0, st>>>(sorted_records, n, k, btot, bytes_out, capacity_bytes, \
-                                                            bucket_start, totals, fmt);
-  MHB_FOR_WR(M)
-#undef M
+    if (int rc = scan32(st, chunk_tot + (u64)q * nc, nc, chunk_off + (u64)q * nc, totals + q, bsum)) return rc;
+  u64 gg = (nc + 7) / 8;
+  if (gg > (u64)sm_count() * 16) gg = (u64)sm_count() * 16;
+  k_s2s_gather<<<(unsigned)gg, 256, 0, st>>>(tmp, chrec, maxb, (u32)nc, chunk_tot, chunk_off, bytes_out, capacity_bytes);
+  CK_LAUNCH();
+  k_bucket_starts<<<64, 256, 0, st>>>(bucket_local, chunk_off, nc, bucket_start);
   CK_LAUNCH();
   k_bucket_finalize<<<1, 1024, 0, st>>>(bucket_start, totals, bucket_table);
   CK_LAUNCH();

@@ -442,9 +442,9 @@ __global__ void __launch_bounds__(G::THREADS, G::CTAS)
     if (s.cta_hist[i]) atomicAdd((unsigned long long *)&mul_hist[i], (unsigned long long)s.cta_hist[i]);
 }
 
-using HcGeomA = HcGeom<256, 11, 3>;
+// 512 threads, 4096 slots, 2 CTAs/SM: geometry B of the sweep in profiles/r2e_* (256 x 2048 x 3 and 1024 x 8192 x 1, at
+// their own and at other slice sizes, were slower)
 using HcGeomB = HcGeom<512, 12, 2>;
-using HcGeomC = HcGeom<1024, 13, 1>;
 
 // per-bucket slice counts: ceil(n_b / T) (0 for an empty bucket)
 __global__ void k_slice_counts(const u64 *__restrict__ bounds, u32 T, u32 *__restrict__ cnt) {
@@ -495,18 +495,6 @@ int scan_counts(cudaStream_t st, const u32 *in, u64 n, u64 *out, u64 *total_dev,
   return MHB_OK;
 }
 
-// MHB_HC_GEOM = A | B | C selects the kernel geometry, MHB_HC_SLICE the records per slice (tuning hooks)
-static int hc_geom() {
-  static const int g = getenv("MHB_HC_GEOM") ? (getenv("MHB_HC_GEOM")[0] == 'A' ? 0 : (getenv("MHB_HC_GEOM")[0] == 'C' ? 2 : 1)) : 1;
-  return g;
-}
-static u32 hc_slice_records() {
-  const u32 def = hc_geom() == 0 ? HcGeomA::SLICE : (hc_geom() == 1 ? HcGeomB::SLICE : HcGeomC::SLICE);
-  static const u32 v = getenv("MHB_HC_SLICE") ? (u32)atoi(getenv("MHB_HC_SLICE")) : 0;
-  return v >= 256 && v <= 64000 ? v : def;
-}
-#define kHcSliceRecords hc_slice_records()
-
 template <class G>
 static int launch_hash_count(cudaStream_t st, const uint2 *recs, const u64 *slice_start, const u64 *n_slices_dev, int m,
                              u32 *misc, u64 *list, u32 *slice_count, u64 *mul_hist) {
@@ -516,7 +504,7 @@ static int launch_hash_count(cudaStream_t st, const uint2 *recs, const u64 *slic
     CK(cudaFuncSetAttribute(k_hash_count<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_hash_count<G>, G::THREADS, smem));
     if (bps < 1) return mhb_set_error(MHB_ERR_CUDA, "hash-count kernel does not fit an SM (%zu B shared memory)", smem);
-    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] hash count: %d threads, %d slots, %zu B smem, %d CTA/SM, slice %u\n", G::THREADS, G::SLOTS, smem, bps, kHcSliceRecords);
+    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] hash count: %d threads, %d slots, %zu B smem, %d CTA/SM, slice %u\n", G::THREADS, G::SLOTS, smem, bps, G::SLICE);
   }
   k_hash_count<G><<<sm_count() * bps, G::THREADS, smem, st>>>(recs, slice_start, n_slices_dev, m, misc, list, slice_count,
                                                              mul_hist, misc + 1);
@@ -532,7 +520,7 @@ struct HcLayout {
 HcLayout hc_layout(uint64_t n, int32_t m) {
   HcLayout L;
   auto pad = [](size_t x) { return (x + 255) & ~(size_t)255; };
-  L.max_slices = n / 256 + 65536 + 2;  // 256 = smallest slice size hc_slice_records() admits
+  L.max_slices = n / HcGeomB::SLICE + 65536 + 2;  // every bucket has ceil(records / SLICE) slices
   L.sort_ws = pad(mhb_sort_workspace_bytes(n, 2));
   size_t p = L.sort_ws;
   L.off_bounds = p;
@@ -606,7 +594,7 @@ extern "C" int mhb_count_solid_hashed(void *stream, uint32_t *recs_a, uint32_t *
   // 2. bucket boundaries, slices per bucket
   k_bucket_bounds<<<(65537 + 255) / 256, 256, 0, st>>>(recs, n, bounds);
   CK_LAUNCH();
-  k_slice_counts<<<65536 / 256, 256, 0, st>>>(bounds, kHcSliceRecords, bcnt);
+  k_slice_counts<<<65536 / 256, 256, 0, st>>>(bounds, HcGeomB::SLICE, bcnt);
   CK_LAUNCH();
   if (int rc = scan_counts(st, bcnt, 65536, slice_off, n_slices_dev, bsum)) return rc;
   CK(cudaMemcpyAsync(slice_off + 65536, n_slices_dev, 8, cudaMemcpyDeviceToDevice, st));
@@ -614,13 +602,7 @@ extern "C" int mhb_count_solid_hashed(void *stream, uint32_t *recs_a, uint32_t *
                                                                             slice_base, slice_bucket);
   CK_LAUNCH();
   // 3. per-slice hash aggregation
-  {
-    int rc;
-    if (hc_geom() == 0) rc = launch_hash_count<HcGeomA>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
-    else if (hc_geom() == 2) rc = launch_hash_count<HcGeomC>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
-    else rc = launch_hash_count<HcGeomB>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist);
-    if (rc) return rc;
-  }
+  if (int rc = launch_hash_count<HcGeomB>(st, recs, slice_start, n_slices_dev, m, misc, list, slice_count, mul_hist)) return rc;
   // 4. offsets + edges (the scan runs over the allocated maximum; unused slice ids hold zero)
   if (int rc = scan_counts(st, slice_count, L.max_slices, slice_dst, n_solid_out, bsum)) return rc;
   k_hash_gather<<<sm_count() * 4, 256, 0, st>>>(list, n_slices_dev, slice_count, slice_dst, slice_base, slice_bucket,

@@ -23,7 +23,7 @@ __device__ __forceinline__ u32 atom_shared_inc_ret(u32 *p) {
 template <int WR>
 struct PartCfg {
   static constexpr int THREADS = 384;
-  static constexpr int IPT = SortCfg3<WR, 0x080>::IPT;
+  static constexpr int IPT = SortCfg3<WR>::IPT;
   static constexpr int TILE = THREADS * IPT;
   static constexpr size_t SMEM = 256 * 8 /*s_base*/ + 4 * 256 * 4 /*s_cnt, s_off, s_cur, s_next*/ + 16 * 4 + (size_t)TILE * WR * 4;
   static constexpr size_t SMEM_OWNER_HIST = SMEM + 16 * 256 * 4;  // + per-owner histograms of the next sort byte

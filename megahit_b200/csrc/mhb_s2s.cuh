@@ -289,180 +289,6 @@ struct EmitAcc {
   u32 bytes, items, tips, large;
 };
 
-// One thread walks the (k-1)-mer group that starts at record i (seq_to_sdbg.cpp:702-789) and either
-// sizes (WRITE=false) or writes (WRITE=true) its SdBG items (sdbg_writer.cpp:25-58).
-template <int W, bool WRITE>
-__device__ __forceinline__ void s2s_group(const u32 *__restrict__ recs, u64 n, u64 i, u32 k, EmitAcc &acc,
-                                          uint8_t *out, u32 *w_count, u32 &ones, u32 fmt = 0) {
-  const u32 WPT = words_per_tip_label(k);
-  u32 r0[W], x[W];
-  ld_rec<W>(recs, i, r0);
-  // pass 1: extent of the group and which a / b have a solid (non-$) edge (:724-738)
-  u32 hsa = 0, hsb = 0;
-  u64 e = i;
-  for (u64 j = i; j < n; ++j) {
-    ld_rec<W>(recs, j, x);
-    if (j > i && diff_km1<W>(r0, x, k)) break;
-    const u32 a = s2s_a<W>(x, k), b = s2s_b<W>(x);
-    if (a != kSentinel && b != kSentinel) {
-      hsa |= 1u << a;
-      hsb |= 1u << b;
-    }
-    e = j + 1;
-  }
-  // pass 2: one item per distinct (a,b) run (:740-786)
-  u32 outputed_b = 0;
-  u64 j = i;
-  u32 cur[W];
-  ld_rec<W>(recs, j, cur);
-  while (j < e) {
-    const u32 a = s2s_a<W>(cur, k), b = s2s_b<W>(cur);
-    u64 t = j + 1;
-    u32 na = 0xFF, nb = 0xFF;  // (a,b) of the next run in this group, if any
-    u32 nx[W];
-    u32 best = cur[W - 1] & 0xFFFFu;  // smallest stored (= largest multiplicity) in the run; the sort ignores it
-    while (t < e) {
-      ld_rec<W>(recs, t, nx);
-      na = s2s_a<W>(nx, k);
-      nb = s2s_b<W>(nx);
-      if (na != a || nb != b) break;
-      best = min(best, nx[W - 1] & 0xFFFFu);
-      ++t;
-    }
-    const bool more = t < e;
-    const bool skip = (a == kSentinel && ((hsb >> b) & 1u)) || (b == kSentinel && ((hsa >> a) & 1u));
-    if (!skip) {
-      const u32 w = (b == kSentinel) ? 0u : (((outputed_b >> b) & 1u) ? b + 5u : b + 1u);
-      // last_a[a] == run end: for a solid `a` the last run with b != $; a non-solid `a` has the single run (a,$)
-      u32 last = 0;
-      if (a != kSentinel) last = (b == kSentinel) ? 1u : ((!more || na != a || nb == kSentinel) ? 1u : 0u);
-      outputed_b |= 1u << b;
-      const u32 mul = 65535u - best;
-      const u32 tip = a == kSentinel ? 1u : 0u;
-      const u32 sz = 2u + (mul > 254u ? 2u : 0u) + (tip ? 4u * WPT : 0u);
-      if (WRITE) {
-        uint16_t *o = reinterpret_cast<uint16_t *>(out + acc.bytes);
-        o[0] = (uint16_t)((w | (last << 4) | (tip << 5)) | ((mul > 255u ? 255u : mul) << 8));
-        u32 p = 1;
-        if (mul > 254u) o[p++] = (uint16_t)mul;
-        if (tip) {
-          for (u32 q = 0; q < WPT; ++q) {
-            u32 lw = pick<W>(cur, q);
-            if (fmt) lw = r2s_label_word(lw, q, (u32)W, k, b);
-            else if (q == (u32)W - 1) lw = (lw & 0xFFFF0000u) | best;  // label = raw words of the run's first sorted record
-            o[p++] = (uint16_t)(lw & 0xFFFFu);
-            o[p++] = (uint16_t)(lw >> 16);
-          }
-        }
-        atomicAdd(&w_count[w], 1u);
-        ones += last;
-      }
-      acc.bytes += sz;
-      acc.items += 1;
-      acc.tips += tip;
-      acc.large += mul > 254u ? 1u : 0u;
-    }
-    j = t;
-    if (more) {
-#pragma unroll
-      for (int q = 0; q < W; ++q) cur[q] = nx[q];
-    }
-  }
-}
-
-static constexpr int kEmitThreads = 256;
-
-// pass 0: per-block totals {bytes, items, tips, large}
-template <int W>
-__global__ void __launch_bounds__(kEmitThreads)
-    k_s2s_size(const u32 *__restrict__ recs, u64 n, u32 k, u64 *btot /*4 per block*/) {
-  __shared__ u32 s_scan[kEmitThreads / 32 + 1];
-  const u64 i = (u64)blockIdx.x * kEmitThreads + threadIdx.x;
-  EmitAcc acc = {0, 0, 0, 0};
-  if (i < n) {
-    bool head = i == 0;
-    if (!head) {
-      u32 a[W], b[W];
-      ld_rec<W>(recs, i - 1, a);
-      ld_rec<W>(recs, i, b);
-      head = diff_km1<W>(a, b, k);
-    }
-    u32 ones = 0;
-    if (head) s2s_group<W, false>(recs, n, i, k, acc, nullptr, nullptr, ones);
-  }
-  u32 t0, t1, t2, t3;
-  block_excl_scan<kEmitThreads>(acc.bytes, s_scan, t0);
-  block_excl_scan<kEmitThreads>(acc.items, s_scan, t1);
-  block_excl_scan<kEmitThreads>(acc.tips, s_scan, t2);
-  block_excl_scan<kEmitThreads>(acc.large, s_scan, t3);
-  if (threadIdx.x == 0) {
-    btot[(u64)blockIdx.x] = t0;
-    btot[(u64)gridDim.x + blockIdx.x] = t1;
-    btot[2ull * gridDim.x + blockIdx.x] = t2;
-    btot[3ull * gridDim.x + blockIdx.x] = t3;
-  }
-}
-
-// pass 1: write items at their final byte offsets; record each bucket's starting prefixes
-template <int W>
-__global__ void __launch_bounds__(kEmitThreads)
-    k_s2s_write(const u32 *__restrict__ recs, u64 n, u32 k, const u64 *btot /*scanned, 4 planes*/,
-                uint8_t *__restrict__ bytes_out, u64 capacity, u64 *bucket_start /*65536*4, init ~0*/,
-                u64 *totals /*16*/, u32 fmt) {
-  __shared__ u32 s_scan[kEmitThreads / 32 + 1];
-  __shared__ u32 s_w[9];
-  if (threadIdx.x < 9) s_w[threadIdx.x] = 0;
-  __syncthreads();
-  const u64 i = (u64)blockIdx.x * kEmitThreads + threadIdx.x;
-  EmitAcc acc = {0, 0, 0, 0};
-  bool head = false;
-  u32 first_word = 0, prev_first_word = 0;
-  if (i < n) {
-    u32 b[W];
-    ld_rec<W>(recs, i, b);
-    first_word = b[0];
-    head = i == 0;
-    if (!head) {
-      u32 a[W];
-      ld_rec<W>(recs, i - 1, a);
-      prev_first_word = a[0];
-      head = diff_km1<W>(a, b, k);
-    }
-    u32 ones = 0;
-    if (head) s2s_group<W, false>(recs, n, i, k, acc, nullptr, nullptr, ones);
-  }
-  u32 t;
-  const u32 e0 = block_excl_scan<kEmitThreads>(acc.bytes, s_scan, t);
-  const u32 e1 = block_excl_scan<kEmitThreads>(acc.items, s_scan, t);
-  const u32 e2 = block_excl_scan<kEmitThreads>(acc.tips, s_scan, t);
-  const u32 e3 = block_excl_scan<kEmitThreads>(acc.large, s_scan, t);
-  u32 ones = 0;
-  if (head) {
-    const u64 nb = gridDim.x;
-    const u64 byte_off = btot[blockIdx.x] + e0;
-    const u64 item_off = btot[nb + blockIdx.x] + e1;
-    const u64 tip_off = btot[2 * nb + blockIdx.x] + e2;
-    const u64 large_off = btot[3 * nb + blockIdx.x] + e3;
-    const u32 bucket = first_word >> 16;
-    if (i == 0 || (prev_first_word >> 16) != bucket) {
-      u64 *bs = bucket_start + 4ull * bucket;
-      bs[0] = byte_off;
-      bs[1] = item_off;
-      bs[2] = tip_off;
-      bs[3] = large_off;
-    }
-    if (byte_off + acc.bytes <= capacity) {
-      EmitAcc wacc = {0, 0, 0, 0};
-      s2s_group<W, true>(recs, n, i, k, wacc, bytes_out + byte_off, s_w, ones, fmt);
-    }
-  }
-  for (int d = 16; d; d >>= 1) ones += __shfl_xor_sync(0xffffffffu, ones, d);
-  if (lane_id() == 0 && ones) atomicAdd((unsigned long long *)&totals[13], (unsigned long long)ones);
-  __syncthreads();
-  if (threadIdx.x < 9 && s_w[threadIdx.x])
-    atomicAdd((unsigned long long *)&totals[4 + threadIdx.x], (unsigned long long)s_w[threadIdx.x]);
-}
-
 // bucket_start holds the prefixes at each non-empty bucket's first item (~0 = empty); turn it into
 // {byte offset, #items, #tips, #large} per bucket using the grand totals for the last bucket.  A bucket's extent ends
 // where the NEXT NON-EMPTY bucket starts.  ONE block of 1024 threads, 64 consecutive buckets per thread: every thread
@@ -542,7 +368,9 @@ struct StagedRecs {
   }
 };
 
-// walk the group starting at record i; returns its end.  WRITE: append item bytes at out + acc.bytes.
+// One thread walks the (k-1)-mer group that starts at record i (seq_to_sdbg.cpp:702-789) and either sizes (WRITE=false)
+// or writes (WRITE=true: item bytes appended at out + acc.bytes) its SdBG items (sdbg_writer.cpp:25-58); returns the
+// group's end.
 template <int W, bool WRITE>
 __device__ __forceinline__ u64 s2s_group2(const StagedRecs<W> &sr, u64 n, u64 i, u32 k, EmitAcc &acc, uint8_t *out,
                                           u32 *w_count, u32 &ones, u32 fmt) {

@@ -1,37 +1,16 @@
-// mhb_sort.cuh -- on-device LSD radix sort of fixed-width records (8-bit digits, one sweep per digit).
+// mhb_sort.cuh -- on-device LSD radix sort of fixed-width records (8-bit digits, one sweep per digit): the pieces the
+// stable sort pass (mhb_sort3.cuh) and the unstable partition pass (mhb_part.cuh) share.
 //
 // Replaces kmlib::kmsort (voutcn/megahit src/kmlib/kmsort.h:43-122, an in-place MSD byte radix +
 // insertion sort run per 16-bit bucket on the CPU) with a stable LSD sort over whole-array passes:
 // same total order on the key (kmsort_selector.cpp:18-27), ties left in input order.
-//
-// One pass = one persistent kernel: every CTA repeatedly claims the next tile (atomic ticket, so tiles
-// start in order), ranks its records by digit with warp match + shared-memory counters, publishes the
-// tile's per-digit counts and resolves its global offsets by decoupled look-back over earlier tiles,
-// reorders the tile in shared memory so that every digit's records are contiguous, and scatters them
-// with coalesced stores.  While the records are in registers the pass also accumulates the histogram
-// of the NEXT pass's digit, so the input is never read just to count.
 #pragma once
 #include "mhb_kernels.cuh"
 
 namespace mhb {
 
-
-// Tile geometry.  CFG selects a (threads, records per thread, CTAs per SM) variant; 0 is the default, the others
-// exist for tuning runs (env MHB_SORT_CFG) and are only instantiated for the narrow records.
-template <int WR, int CFG = 0>
-struct SortCfg {
-  static constexpr int THREADS = CFG == 1 ? 256 : (CFG == 2 ? 256 : (CFG == 3 ? 512 : 384));
-  static constexpr int MIN_BLOCKS = CFG == 1 ? 3 : (CFG == 2 ? 4 : 2);
-  static constexpr int IPT_NARROW = CFG == 1 ? 18 : (CFG == 2 ? 12 : (CFG == 3 ? 14 : 18));
-  static constexpr int IPT = WR <= 2 ? IPT_NARROW
-                                     : (WR <= 3 ? (IPT_NARROW * 2) / 3 : (WR <= 4 ? 10 : (WR <= 6 ? 6 : (WR <= 9 ? 4 : 2))));
-  static constexpr int TILE = THREADS * IPT;
-  static constexpr int NW = THREADS / 32;
-  static constexpr size_t SMEM = (size_t)(NW * 256 + 256 + 256 + 8) * 4 + 256 * 8 + (size_t)TILE * WR * 4;
-};
-
 // exclusive scan of a 256-bin histogram (one block of 256 threads) -> where each digit's records start, as a
-// BYTE ADDRESS: out + offset * rec_bytes.  (The pass kernel takes per-digit addresses so that the same kernel can
+// BYTE ADDRESS: out + offset * rec_bytes.  (The pass kernels take per-digit addresses so that the partition pass can
 // scatter straight into other GPUs' memory, see mhb_partition_scatter.)
 __global__ void k_hist_scan256(const u64 *hist, u64 *bin_addr, u64 out_addr, u32 rec_bytes) {
   __shared__ u64 s[256];
@@ -71,204 +50,6 @@ __device__ __forceinline__ u32 rec_digit(const u32 (&r)[WR], u32 widx, u32 bsel)
   else if constexpr (WR == 2) w = widx ? r[1] : r[0];
   else w = pick<WR>(r, widx);
   return __byte_perm(w, 0, 0x4440u | bsel);
-}
-
-static constexpr int kLbWindow = 4;  // look-back descriptors fetched per round trip
-
-// OWNER_LUT: the digit is digit_lut[record byte] instead of the byte itself (multi-GPU partition pass: the digit is the
-// owning rank, so each tile leaves ONE long contiguous run per destination GPU instead of one short run per byte value
-// - NVLink-friendly stores; the full sort on the owner re-sorts that byte anyway).
-template <int WR, int CFG = 0, bool OWNER_LUT = false>
-__global__ void __launch_bounds__(SortCfg<WR, CFG>::THREADS, SortCfg<WR, CFG>::MIN_BLOCKS)
-    k_radix_pass(const u32 *__restrict__ in, u64 n, u32 num_tiles, int byte_idx,
-                 const u64 *__restrict__ bin_addr /*byte address of each digit's first output record*/,
-                 u64 *lookback, u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch,
-                 const uint8_t *__restrict__ digit_lut = nullptr) {
-  using C = SortCfg<WR, CFG>;
-  constexpr int THREADS = C::THREADS, IPT = C::IPT, TILE = C::TILE, NW = C::NW;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  u64 *s_glob = reinterpret_cast<u64 *>(smem_raw);          // 256: byte address of the digit's slot for tile position 0
-  u32 *s_warp_hist = reinterpret_cast<u32 *>(s_glob + 256);  // NW*256
-  u32 *s_bin_start = s_warp_hist + NW * 256;                 // 256
-  u32 *s_next = s_bin_start + 256;                           // 256
-  u32 *s_misc = s_next + 256;                                // 8 (ticket)
-  u32 *s_recs = s_misc + 8;                                  // TILE*WR (16-byte aligned)
-  __shared__ u32 s_scan[THREADS / 32 + 1];
-
-  const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const u32 lt_mask = lanemask_lt();
-  const u64 ep = lb_epoch(epoch);
-  const u32 widx = (u32)(WR - 1 - (byte_idx >> 2)), bsel = (u32)(byte_idx & 3);
-  const u32 nwidx = (u32)(WR - 1 - (next_byte >> 2)), nbsel = (u32)(next_byte & 3);
-  u32 *my_hist = s_warp_hist + warp * 256;
-
-  for (int i = tid; i < 256; i += THREADS) s_next[i] = 0;
-  __shared__ uint8_t s_lut[OWNER_LUT ? 256 : 1];
-  if constexpr (OWNER_LUT) {
-    for (int i = tid; i < 256; i += THREADS) s_lut[i] = digit_lut[i];
-    __syncthreads();
-  }
-
-  while (true) {
-    if (tid == 0) s_misc[0] = atomicAdd(tile_counter, 1u);
-    for (int i = tid; i < NW * 256; i += THREADS) s_warp_hist[i] = 0;
-    __syncthreads();
-    const u32 tile = s_misc[0];
-    if (tile >= num_tiles) break;
-    const u64 tile_base = (u64)tile * TILE;
-    const u32 valid = (u32)((n - tile_base) < (u64)TILE ? (n - tile_base) : (u64)TILE);
-
-    // ---- load (warp-striped: slot i of lane l = warp chunk[i*32 + l]) ----
-    u32 r[IPT][WR];
-    const u64 warp_base = tile_base + (u64)warp * 32 * IPT + lane;
-    if (tile_base + TILE <= n) {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) ld_rec<WR>(in, warp_base + (u64)i * 32, r[i]);
-    } else {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        const u64 idx = warp_base + (u64)i * 32;
-        if (idx < n) {
-          ld_rec<WR>(in, idx, r[i]);
-        } else {
-#pragma unroll
-          for (int j = 0; j < WR; ++j) r[i][j] = 0xFFFFFFFFu;  // padding sorts to the very end of the tile
-        }
-      }
-    }
-
-    // ---- rank inside the warp.  peers = lanes holding the same digit, from eight ballots (one per digit bit):
-    // MATCH.ANY costs time proportional to the number of distinct digits in the warp (measured: 41 % of all
-    // stall samples on random digits), eight votes cost the same for every distribution.  The highest peer
-    // lane bumps the warp's digit counter.
-    u32 rk[IPT];  // digit << 16 | rank within (warp, digit)
-#pragma unroll
-    for (int i = 0; i < IPT; ++i) {
-      u32 d = rec_digit<WR>(r[i], widx, bsel);
-      if constexpr (OWNER_LUT) d = s_lut[d];
-      u32 peers = 0xffffffffu;
-#pragma unroll
-      for (int bit = 0; bit < 8; ++bit) {
-        u32 mask;
-        asm("{\n\t.reg .pred p;\n\t.reg .b32 t;\n\tand.b32 t, %1, %2;\n\tsetp.ne.u32 p, t, 0;\n\t"
-            "vote.sync.ballot.b32 %0, p, 0xffffffff;\n\t@!p not.b32 %0, %0;\n\t}"
-            : "=r"(mask)
-            : "r"(d), "r"(1u << bit));
-        peers &= mask;
-      }
-      const u32 leader = 31u - __clz(peers);
-      u32 old = 0;
-      if (lane == leader) {
-        old = my_hist[d];
-        my_hist[d] = old + __popc(peers);
-      }
-      __syncwarp();
-      old = __shfl_sync(0xffffffffu, old, leader);
-      rk[i] = (d << 16) | (old + __popc(peers & lt_mask));
-    }
-    __syncthreads();
-
-    // ---- per digit: prefix over warps, tile total, local start; publish the tile's counts ----
-    u32 total = 0;
-    if (tid < 256) {
-#pragma unroll
-      for (int w = 0; w < NW; ++w) {
-        const u32 c = s_warp_hist[w * 256 + tid];
-        s_warp_hist[w * 256 + tid] = total;
-        total += c;
-      }
-    }
-    u32 tile_total;
-    const u32 excl = block_excl_scan<THREADS>(total, s_scan, tile_total);
-    // padding records all carry digit 255 and are not real: exclude them from what we publish
-    const u64 pub = (u64)total - ((tid == 255) ? (u64)(TILE - valid) : 0ull);
-    u64 *my = lookback + (u64)tile * 256 + tid;
-    u64 win[kLbWindow];
-    if (tid < 256) {
-      s_bin_start[tid] = excl;
-      st_relaxed(my, (tile == 0 ? kLbInclusive : kLbPartial) | ep | pub);
-      // first window of predecessor descriptors: in flight while the tile is reordered below
-#pragma unroll
-      for (int j = 0; j < kLbWindow; ++j)
-        win[j] = (tile > (u32)j) ? ld_relaxed(lookback + (u64)(tile - 1 - j) * 256 + tid) : 0ull;
-    }
-    __syncthreads();
-    // fold the digit's local start into every warp's prefix: warp_hist[w][d] = position of the warp's first d
-    for (int i = tid; i < NW * 256; i += THREADS) s_warp_hist[i] += s_bin_start[i & 255];
-    __syncthreads();
-
-    // ---- reorder in shared memory: every digit's records become contiguous, input order kept ----
-#pragma unroll
-    for (int i = 0; i < IPT; ++i) {
-      const u32 d = rk[i] >> 16;
-      const u32 pos = my_hist[d] + (rk[i] & 0xFFFFu);
-      st_rec<WR>(s_recs, pos, r[i]);
-    }
-
-    // ---- global offsets by decoupled look-back, kLbWindow descriptors per round trip ----
-    if (tid < 256) {
-      u64 prefix = 0;
-      if (tile > 0) {
-        u32 p = tile - 1;  // descriptor win[0] belongs to tile p
-        bool done = false;
-        while (!done) {
-#pragma unroll
-          for (int j = 0; j < kLbWindow; ++j) {
-            if (done) break;
-            u64 v = win[j];
-            const u64 *pp = lookback + (u64)(p - j) * 256 + tid;
-            while ((v & kLbStatusMask) == 0 || (v & lb_epoch(255)) != ep) v = ld_relaxed(pp);
-            prefix += v & kLbValueMask;
-            if ((v & kLbStatusMask) == kLbInclusive || p == (u32)j) done = true;
-          }
-          if (!done) {
-            p -= kLbWindow;
-#pragma unroll
-            for (int j = 0; j < kLbWindow; ++j)
-              win[j] = (p >= (u32)j) ? ld_relaxed(lookback + (u64)(p - j) * 256 + tid) : 0ull;
-          }
-        }
-        st_relaxed(my, kLbInclusive | ep | (prefix + pub));
-      }
-      s_glob[tid] = bin_addr[tid] + (prefix - (u64)excl) * (u64)(WR * 4);  // may address another GPU's memory
-    }
-    __syncthreads();
-
-    // ---- coalesced scatter + next digit's histogram ----
-    if (next_hist) {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        const u32 p = (u32)i * THREADS + tid;
-        if (p < valid) {
-          u32 q[WR];
-          ld_rec<WR>(s_recs, p, q);
-          u32 dd = rec_digit<WR>(q, widx, bsel);
-          if constexpr (OWNER_LUT) dd = s_lut[dd];
-          st_rec<WR>(reinterpret_cast<u32 *>(s_glob[dd] + (u64)p * (WR * 4)), 0, q);
-          atomicAdd(&s_next[rec_digit<WR>(q, nwidx, nbsel)], 1u);
-        }
-      }
-    } else {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        const u32 p = (u32)i * THREADS + tid;
-        if (p < valid) {
-          u32 q[WR];
-          ld_rec<WR>(s_recs, p, q);
-          u32 dd = rec_digit<WR>(q, widx, bsel);
-          if constexpr (OWNER_LUT) dd = s_lut[dd];
-          st_rec<WR>(reinterpret_cast<u32 *>(s_glob[dd] + (u64)p * (WR * 4)), 0, q);
-        }
-      }
-    }
-    __syncthreads();
-  }
-
-  if (next_hist) {
-    __syncthreads();
-    for (int i = tid; i < 256; i += THREADS)
-      if (s_next[i]) atomicAdd((unsigned long long *)&next_hist[i], (unsigned long long)s_next[i]);
-  }
 }
 
 }  // namespace mhb

@@ -1,75 +1,43 @@
-// mhb_sort3.cuh -- radix pass v3: the same one-sweep LSD pass as k_radix_pass (mhb_sort.cuh: ticketed tiles, warp
-// ranking, decoupled look-back, shared-memory reorder, coalesced scatter, next digit's histogram fused into the
-// scatter) rebuilt around the instruction budget.  v2 was issue-bound at ~125 thread-instructions per record
-// (profiles/r1_radix_v2_*.txt: 24 % issue-active with 2 CTAs/SM, DRAM traffic 1.01x algorithmic), of which only ~26
-// are the eight ballots.  v3 removes what surrounded them:
-//   * one tile ticket is prefetched a whole tile ahead (the global atomic's latency is never exposed);
+// mhb_sort3.cuh -- the stable radix pass.  One pass = one persistent kernel: every CTA repeatedly claims the next tile
+// (atomic ticket, so tiles start in order), ranks its records by digit with warp ballots and per-warp shared-memory
+// counters, publishes the tile's per-digit counts and resolves its global offsets by decoupled look-back over earlier
+// tiles, reorders the tile in shared memory so that every digit's records are contiguous, and scatters them with
+// coalesced stores.  While the records are in registers the pass also accumulates the histogram of the NEXT pass's
+// digit, so the input is never read just to count.
+//
+// The round-1 pass was issue-bound at ~125 thread-instructions per record (profiles/r1_radix_v2_*.txt: 24 %
+// issue-active with 2 CTAs/SM, DRAM traffic 1.01x algorithmic), of which only ~26 were the eight ballots.  This one
+// removes what surrounded them:
+//   * the next tile's ticket is requested a whole tile ahead (the global atomic's latency is never exposed);
 //   * per-warp digit counters are read by ALL lanes before the leader bumps them (no shuffle, no divergent load);
 //   * the prefix over warps, the tile scan and the fold of the digit's start run as ONE pass of 256 threads
 //     (6 block barriers per tile instead of 9, no separate fold loop, no s_bin_start array);
+//   * a tile's digit counts are histogrammed and published right after its load, before ranking (early publish);
 //   * full tiles take a scatter path without per-record bounds checks;
 //   * counters are cleared with 128-bit stores while the scatter's global stores are in flight.
-// RANK selects how a lane finds the lanes holding the same digit:
-//   0 = eight vote.ballot (constant cost, no shared-memory traffic),
-//   1 = shared-memory OR-match: red.or the lane bit into a per-warp {mask,count} slot, read both back with one
-//       64-bit load (2 shared-memory instructions instead of ~26 ALU ones; cost depends on digit collisions).
+// Measured on B200, 1.23 G 8-byte records, this pass takes 6.44 ms; other tile shapes, shared-memory OR-match ranking,
+// register prefetch of the next tile, batched shared-memory loads, wider or narrower look-back windows, compact
+// look-back descriptors and two-stream ranking were all slower (profiles/r1d_sort_sweep.txt, profiles/r2a_sort_sweep.json).
 #pragma once
 #include "mhb_sort.cuh"
 
 namespace mhb {
 
-// CFG is a bit field so that single design choices can be A/B-ed on the GPU (scripts/sort_sweep.py):
-//   bits 0-1  geometry: 0 = 384 thr x 18 rec (2 CTA/SM), 1 = 384 x 20, 2 = 256 x 18 (3 CTA/SM), 3 = 384 x 16
-//   bit  2    ranking: 0 = eight ballots, 1 = shared-memory OR-match
-//   bit  3    register prefetch of the next tile
-//   bits 4-5  look-back descriptors per round trip after the first window: 2, 4, 8, 1
-//   bit  6    reorder / scatter with batched shared-memory loads (asm stores without memory clobber)
-//   bit  7    early publish: a tile's digit counts are histogrammed and published right after its load, before ranking
-//   bit  8    first (prefetched) look-back window of 1 descriptor instead of 2
-//   bits 9-10 high-occupancy geometries (override bits 0-1): 1 = 256 thr x 12 rec, 4 CTA/SM; 2 = 512 x 12, 2 CTA/SM
-//   bit  11   (with bit 3) the prefetch is issued after the look-back, at the start of the scatter, instead of before it
-//   bit  15   compact look-back descriptors: the partial counts of 4 consecutive tiles share one 16-byte word per digit
-//             (one load examines 4 predecessors), the 64-bit inclusive prefixes live in a separate array
-//   bit  16   ranking in two interleaved streams per warp (records 0..H-1 and H..IPT-1 with separate counter rows):
-//             two independent shared-memory dependency chains instead of one
-//   bit  13   batched loads in the reorder only; bit 14: in the warp-base loop only (bit 6 = both + the asm scatter)
-//   bit  12   (with bit 7) the scan over the digit totals also runs early, on the early histogram: one barrier and the
-//             per-warp total loop leave the critical path between ranking and the reorder
-// Measured on B200, 1.23 G 8-byte records, ms per pass (profiles/r1d_sort_sweep.txt): v2 7.24; v3 base 6.93;
-// + prefetch 6.72; + early publish 6.44 (default); wider look-back windows (8, 16) 6.8-7.6; batched loads 7.1-7.3;
-// OR-match ranking 7.3.
-template <int WR, int CFG>
+// Tile geometry: 384 threads, 2 CTAs/SM, records per thread by width so that a tile's records fill ~55 KB of shared memory
+template <int WR>
 struct SortCfg3 {
-  static constexpr int GEOM = CFG & 3;
-  static constexpr int GEOMX = (CFG >> 9) & 3;
-  static constexpr int RANK = (CFG >> 2) & 1;
-  static constexpr bool PREFETCH = (CFG >> 3) & 1;
-  static constexpr int LBW = ((CFG >> 4) & 3) == 3 ? 1 : (2 << ((CFG >> 4) & 3));
-  static constexpr bool BATCH = (CFG >> 6) & 1;
-  static constexpr bool BATCH_R = BATCH || ((CFG >> 13) & 1);
-  static constexpr bool BATCH_P = BATCH || ((CFG >> 14) & 1);
-  static constexpr bool EARLY = (CFG >> 7) & 1;
-  static constexpr int LB1 = ((CFG >> 8) & 1) ? 1 : 2;
-  static constexpr bool LATEPF = (CFG >> 11) & 1;
-  static constexpr bool ESCAN = EARLY && ((CFG >> 12) & 1);
-  static constexpr bool CDESC = EARLY && ((CFG >> 15) & 1);
-  static constexpr bool RANK2 = RANK == 0 && ((CFG >> 16) & 1);
-  static constexpr int THREADS = GEOMX == 1 ? 256 : (GEOMX == 2 ? 512 : (GEOM == 2 ? 256 : 384));
-  static constexpr int MIN_BLOCKS = GEOMX == 1 ? 4 : (GEOMX == 2 ? 2 : (THREADS == 256 ? 3 : 2));
-  static constexpr int IPT_NARROW = GEOMX ? 12 : (GEOM == 1 ? 20 : (GEOM == 3 ? 16 : 18));
-  static constexpr int IPT = WR <= 2 ? IPT_NARROW
-                                     : (WR <= 3 ? (IPT_NARROW * 2) / 3 : (WR <= 4 ? 10 : (WR <= 6 ? 6 : (WR <= 9 ? 4 : 2))));
+  static constexpr int THREADS = 384;
+  static constexpr int MIN_BLOCKS = 2;
+  static constexpr int IPT = WR <= 2 ? 18 : (WR <= 3 ? 12 : (WR <= 4 ? 10 : (WR <= 6 ? 6 : (WR <= 9 ? 4 : 2))));
   static constexpr int TILE = THREADS * IPT;
   static constexpr int NW = THREADS / 32;
-  static constexpr int NROW = RANK2 ? 2 * NW : NW;   // counter rows: one per warp, or one per (warp, stream)
-  static constexpr int HA = RANK2 ? (IPT + 1) / 2 : IPT;  // records of the first stream
-  static constexpr int CSTRIDE = RANK == 1 ? 2 : 1;  // words per counter slot ({mask,count} when OR-matching)
-  static constexpr size_t SMEM = 256 * 8 /*s_glob*/ + (size_t)NROW * 256 * CSTRIDE * 4 /*counters*/ + 256 * 4 /*s_next*/ +
+  static constexpr int LBW = 2;  // look-back descriptors fetched per round trip; the first window is fetched before the reorder
+  static constexpr size_t SMEM = 256 * 8 /*s_glob*/ + (size_t)NW * 256 * 4 /*counters*/ + 256 * 4 /*s_next*/ +
                                  256 * 4 /*s_early*/ + 16 * 4 /*misc*/ + (size_t)TILE * WR * 4;
 };
 
-// the next tile's records are requested as soon as this tile's registers are free (after the shared-memory reorder), so
-// the DRAM latency of the loads hides behind the look-back and the scatter.  asm volatile pins the loads there.
+// a tile's record loads, issued where they stand: asm volatile keeps the compiler from moving them past the shared-memory
+// work around them
 template <int WR>
 __device__ __forceinline__ void ld_rec_pinned(const u32 *base, u64 idx, u32 (&r)[WR]) {
   const u32 *p = base + idx * WR;
@@ -88,11 +56,11 @@ __device__ __forceinline__ void ld_rec_pinned(const u32 *base, u64 idx, u32 (&r)
   }
 }
 
-// Stores/reductions issued from the unrolled reorder / scatter loops.  As plain C++ they would be generic-address
-// stores that may alias shared memory, which forces the compiler to serialise "load record i+1" behind "store record
-// i"; as asm without a memory clobber the shared-memory loads of a whole chunk are issued back to back (the kernel is
+// Stores/reductions issued from the unrolled reorder / scatter loops of the partition pass (mhb_part.cuh).  As plain
+// C++ they would be generic-address stores that may alias shared memory, which forces the compiler to serialise "load
+// record i+1" behind "store record i"; as asm without a memory clobber the shared-memory loads of a whole chunk are issued back to back (the kernel is
 // latency-bound at 2 CTAs/SM, so every exposed 30-cycle LDS round trip counts).  Nothing read inside those loops is
-// written by them: s_recs/s_glob are complete before the barrier that precedes the scatter.
+// written by them: the reordered records and the digit bases are complete before the barrier that precedes the scatter.
 template <int WR>
 __device__ __forceinline__ void st_global_rec(u64 addr, const u32 (&q)[WR]) {
   if constexpr (WR % 4 == 0) {
@@ -107,15 +75,6 @@ __device__ __forceinline__ void st_global_rec(u64 addr, const u32 (&q)[WR]) {
     for (int j = 0; j < WR; ++j) asm volatile("st.global.u32 [%0], %1;" ::"l"(addr + 4 * j), "r"(q[j]));
   }
 }
-__device__ __forceinline__ void st_relaxed_u32(u32 *p, u32 v) {
-  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint4 ld_relaxed_v4(const u32 *p) {
-  uint4 v;
-  asm volatile("ld.relaxed.gpu.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ u32 pick4(const uint4 &v, u32 e) { return e == 0 ? v.x : (e == 1 ? v.y : (e == 2 ? v.z : v.w)); }
 __device__ __forceinline__ void red_shared_inc(u32 *p) {
   asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(smem_u32(p)));
 }
@@ -196,50 +155,34 @@ __device__ unsigned long long g_sort_timeline_rows = 0;
 #define MHB_TL_FLUSH() ((void)0)
 #endif
 
-template <int WR, int CFG, bool OWNER_LUT = false, bool HAS_NEXT = true>
-__global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>::MIN_BLOCKS)
+template <int WR, bool HAS_NEXT = true>
+__global__ void __launch_bounds__(SortCfg3<WR>::THREADS, SortCfg3<WR>::MIN_BLOCKS)
     k_radix_pass3(const u32 *__restrict__ in, u64 n, u32 num_tiles, int byte_idx,
                   const u64 *__restrict__ bin_addr /*byte address of each digit's first output record*/, u64 *lookback,
-                  u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch,
-                  const uint8_t *__restrict__ digit_lut = nullptr) {
-  using C = SortCfg3<WR, CFG>;
-  constexpr int THREADS = C::THREADS, IPT = C::IPT, TILE = C::TILE, RANK = C::RANK, CS = C::CSTRIDE;
-  constexpr int CO = CS - 1;  // word offset of the count inside a slot
-  constexpr bool PREFETCH = C::PREFETCH;
-  constexpr int LBW = C::LBW, LB1 = C::LB1;
-  constexpr bool CDESC = C::CDESC, RANK2 = C::RANK2;
-  constexpr int NROW = C::NROW, HA = C::HA;
-  constexpr bool BATCH = C::BATCH, BATCH_R = C::BATCH_R, BATCH_P = C::BATCH_P, EARLY = C::EARLY, LATEPF = C::LATEPF, ESCAN = C::ESCAN;
+                  u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch) {
+  using C = SortCfg3<WR>;
+  constexpr int THREADS = C::THREADS, IPT = C::IPT, TILE = C::TILE, NW = C::NW, LBW = C::LBW;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   u64 *s_glob = reinterpret_cast<u64 *>(smem_raw);        // 256: byte address of the digit's slot for tile position 0
-  u32 *s_cnt = reinterpret_cast<u32 *>(s_glob + 256);     // NROW * 256 * CS
-  u32 *s_next = s_cnt + NROW * 256 * CS;                  // 256
-  u32 *s_early = s_next + 256;                            // 256: tile digit counts taken right after the load (EARLY)
+  u32 *s_cnt = reinterpret_cast<u32 *>(s_glob + 256);     // NW * 256
+  u32 *s_next = s_cnt + NW * 256;                         // 256
+  u32 *s_early = s_next + 256;                            // 256: tile digit counts taken right after the load
   u32 *s_misc = s_early + 256;                            // 16: [0] ticket, [4..12] scan
   u32 *s_recs = s_misc + 16;                              // TILE * WR (16-byte aligned)
-  __shared__ uint8_t s_lut[OWNER_LUT ? 256 : 1];
 
   const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const u32 lt_mask = lanemask_lt();
   const u32 widx = (u32)(WR - 1 - (byte_idx >> 2)), bsel = (u32)(byte_idx & 3);
   const u32 nwidx = (u32)(WR - 1 - (next_byte >> 2)), nbsel = (u32)(next_byte & 3);
-  u32 *my_cnt = s_cnt + (RANK2 ? 2 * warp : warp) * 256 * CS;  // RANK2: the second stream's row follows at +256
-  // compact descriptors (CDESC): part[(tile >> 2) * 256 + digit][tile & 3] = status<<30 | epoch<<22 | count behind the
-  // inclusive array; status 1 = count valid, 3 = count valid and the tile's inclusive prefix is in lookback[]
-  u32 *part = reinterpret_cast<u32 *>(lookback + (u64)num_tiles * 256);
-  const u32 ep22 = (epoch & 255u) << 22;
+  u32 *my_cnt = s_cnt + warp * 256;
   MHB_TL_DECL
 
   for (int i = tid; i < 256; i += THREADS) s_next[i] = 0;
   for (int i = tid; i < 256; i += THREADS) s_early[i] = 0;
-  for (int i = tid; i < NROW * 256 * CS; i += THREADS) s_cnt[i] = 0;
-  if constexpr (OWNER_LUT) {
-    for (int i = tid; i < 256; i += THREADS) s_lut[i] = digit_lut[i];
-  }
+  for (int i = tid; i < NW * 256; i += THREADS) s_cnt[i] = 0;
   if (tid == 0) s_misc[0] = atomicAdd(tile_counter, 1u);
   __syncthreads();
   u32 tile = s_misc[0];
-  const u32 pad_digit = OWNER_LUT ? (u32)s_lut[255] : 255u;  // digit the 0xFF padding records of a ragged tile get
 
   // ---- load (warp-striped: slot i of lane l = warp chunk[i*32 + l]) ----
   u32 r[IPT][WR];
@@ -262,9 +205,6 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
       }
     }
   };
-  if constexpr (PREFETCH) {
-    if (tile < num_tiles) load_tile(tile);
-  }
 
   while (tile < num_tiles) {
     // ticket of the NEXT tile: requested now, stored to shared memory just before this tile's last barrier, so the
@@ -277,11 +217,11 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
     const bool full = tile_base + TILE <= n;
     const u32 valid = full ? (u32)TILE : (u32)(n - tile_base);
 
-    if constexpr (!PREFETCH) load_tile(tile);
+    load_tile(tile);
 
-    // ---- EARLY: histogram the tile's digits and publish the counts now, a whole rank phase before the tile needs its
-    // predecessors: when the following tiles look back, this descriptor is already there (no spinning on "invalid")
-    u32 e_total = 0, e_excl = 0;
+    // ---- early publish: histogram the tile's digits and publish the counts now, a whole rank phase before the tile
+    // needs its predecessors: when the following tiles look back, this descriptor is already there (no spinning on
+    // "invalid")
 #ifdef MHB_SORT_TIMELINE
     if (tid == 0) {  // first use of the tile's records: the wait for the loads ends here
       volatile u32 sink = r[0][0];
@@ -289,40 +229,22 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
       tl_v[0] = clock64() - tl_t0;
     }
 #endif
-    if constexpr (EARLY) {
 #pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        u32 d = rec_digit<WR>(r[i], widx, bsel);
-        if constexpr (OWNER_LUT) d = s_lut[d];
-        red_shared_inc(&s_early[d]);
-      }
-      __syncthreads();
-      if (tid < 256) {
-        e_total = s_early[tid];
-        const u32 c = e_total - ((tid == pad_digit) ? (u32)(TILE - valid) : 0u);
-        if constexpr (CDESC) {
-          if (tile == 0) st_relaxed(lookback + tid, kLbInclusive | lb_epoch(epoch) | (u64)c);  // before the flag below
-          st_relaxed_u32(part + ((u64)(tile >> 2) * 256 + tid) * 4 + (tile & 3u), ((tile == 0 ? 3u : 1u) << 30) | ep22 | c);
-        } else {
-          st_relaxed(lookback + (u64)tile * 256 + tid, (tile == 0 ? kLbInclusive : kLbPartial) | lb_epoch(epoch) | (u64)c);
-        }
-        if constexpr (ESCAN) {
-          u32 inc = e_total;
-#pragma unroll
-          for (int dd = 1; dd < 32; dd <<= 1) {
-            const u32 t = __shfl_up_sync(0xffffffffu, inc, dd);
-            if (lane >= (u32)dd) inc += t;
-          }
-          if (lane == 31) s_misc[4 + warp] = inc;  // read after B1
-          e_excl = inc - e_total;
-        }
-      }
+    for (int i = 0; i < IPT; ++i) red_shared_inc(&s_early[rec_digit<WR>(r[i], widx, bsel)]);
+    __syncthreads();
+    if (tid < 256) {
+      // padding records all carry digit 255 and are not real: exclude them from what we publish
+      const u32 c = s_early[tid] - ((tid == 255) ? (u32)(TILE - valid) : 0u);
+      st_relaxed(lookback + (u64)tile * 256 + tid, (tile == 0 ? kLbInclusive : kLbPartial) | lb_epoch(epoch) | (u64)c);
     }
 
     MHB_TL_MARK(1);
-    // ---- rank inside the warp: rk = rank among the warp's records with the same digit << 8 | digit ----
+    // ---- rank inside the warp: rk = rank among the warp's records with the same digit << 8 | digit.  The lanes
+    // holding the same digit come from eight ballots, one per digit bit: constant cost, no shared-memory traffic ----
     u32 rk[IPT];
-    auto ballot_peers = [&](u32 d) {
+#pragma unroll
+    for (int i = 0; i < IPT; ++i) {
+      const u32 d = rec_digit<WR>(r[i], widx, bsel);
       u32 peers = 0xffffffffu;
 #pragma unroll
       for (int bit = 0; bit < 8; ++bit) {
@@ -333,199 +255,76 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
             : "r"(d), "r"(1u << bit));
         peers &= mask;
       }
-      return peers;
-    };
-    if constexpr (RANK2) {
-      // two independent streams: record j of the first half and record HA + j of the second are ranked together, each
-      // against its own counter row, so the two load -> store -> load chains through shared memory overlap
-#pragma unroll
-      for (int j = 0; j < HA; ++j) {
-        const bool hasb = HA + j < IPT;
-        u32 da = rec_digit<WR>(r[j], widx, bsel);
-        u32 db = hasb ? rec_digit<WR>(r[hasb ? HA + j : j], widx, bsel) : 0u;
-        if constexpr (OWNER_LUT) {
-          da = s_lut[da];
-          db = s_lut[db];
-        }
-        const u32 pa = ballot_peers(da);
-        const u32 pb = hasb ? ballot_peers(db) : 0u;
-        volatile u32 *sla = my_cnt + da;
-        volatile u32 *slb = my_cnt + 256 + db;
-        const u32 olda = *sla;
-        const u32 oldb = hasb ? *slb : 0u;
-        __syncwarp();
-        const u32 ba = __popc(pa & lt_mask), bb = __popc(pb & lt_mask);
-        if ((pa >> lane) <= 1u) *sla = olda + ba + 1u;
-        if (hasb && (pb >> lane) <= 1u) *slb = oldb + bb + 1u;
-        __syncwarp();
-        rk[j] = ((olda + ba) << 8) | da;
-        if (hasb) rk[hasb ? HA + j : j] = ((oldb + bb) << 8) | db;
-      }
-    } else {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        u32 d = rec_digit<WR>(r[i], widx, bsel);
-        if constexpr (OWNER_LUT) d = s_lut[d];
-        u32 peers, old, below;
-        if constexpr (RANK == 0) {
-          peers = ballot_peers(d);
-          volatile u32 *slot = my_cnt + d;
-          old = *slot;  // every lane reads the running count before the leader bumps it
-          __syncwarp();
-          below = __popc(peers & lt_mask);
-          if ((peers >> lane) <= 1u) *slot = old + below + 1u;  // highest peer lane: below + 1 = popc(peers)
-          __syncwarp();
-        } else {
-          u32 *slot = my_cnt + d * 2;
-          const u32 sa = smem_u32(slot);
-          asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(sa), "r"(1u << lane) : "memory");
-          __syncwarp();
-          asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(peers), "=r"(old) : "r"(sa) : "memory");
-          __syncwarp();
-          below = __popc(peers & lt_mask);
-          if ((peers >> lane) <= 1u)  // highest peer lane: clear the mask, bump the count (below + 1 = popc(peers))
-            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(sa), "r"(0u), "r"(old + below + 1u) : "memory");
-          __syncwarp();
-        }
-        rk[i] = ((old + below) << 8) | d;
-      }
+      volatile u32 *slot = my_cnt + d;
+      const u32 old = *slot;  // every lane reads the running count before the leader bumps it
+      __syncwarp();
+      const u32 below = __popc(peers & lt_mask);
+      if ((peers >> lane) <= 1u) *slot = old + below + 1u;  // highest peer lane: below + 1 = popc(peers)
+      __syncwarp();
+      rk[i] = ((old + below) << 8) | d;
     }
     __syncthreads();  // B1: all warps' counters final
     MHB_TL_MARK(2);
 
-    // ---- per digit (threads 0..255): tile total, scan over digits, warp bases; publish; first look-back window ----
+    // ---- per digit (threads 0..255): tile total, scan over digits, warp bases; first look-back window ----
     u32 total = 0, excl = 0;
-    if constexpr (ESCAN) {
-      total = e_total;
-      excl = e_excl;
-    } else {
-      if (tid < 256) {
+    if (tid < 256) {
 #pragma unroll
-        for (int w = 0; w < NROW; ++w) total += s_cnt[(w * 256 + tid) * CS + CO];
-        u32 inc = total;
+      for (int w = 0; w < NW; ++w) total += s_cnt[w * 256 + tid];
+      u32 inc = total;
 #pragma unroll
-        for (int dd = 1; dd < 32; dd <<= 1) {
-          const u32 t = __shfl_up_sync(0xffffffffu, inc, dd);
-          if (lane >= (u32)dd) inc += t;
-        }
-        if (lane == 31) s_misc[4 + warp] = inc;
-        excl = inc - total;
+      for (int dd = 1; dd < 32; dd <<= 1) {
+        const u32 t = __shfl_up_sync(0xffffffffu, inc, dd);
+        if (lane >= (u32)dd) inc += t;
       }
-      __syncthreads();  // B2
+      if (lane == 31) s_misc[4 + warp] = inc;
+      excl = inc - total;
     }
+    __syncthreads();  // B2
     u32 pub = 0;
-    u64 win[LB1];
-    uint4 cwin = make_uint4(0u, 0u, 0u, 0u);
+    u64 win[LBW];
     if (tid == 0) s_misc[0] = next_ticket;  // requested a whole rank phase ago: no wait
     if (tid < 256) {
 #pragma unroll
       for (int w = 0; w < 7; ++w) excl += (warp > (u32)w) ? s_misc[4 + w] : 0u;
-      // padding records all carry digit 255 and are not real: exclude them from what we publish
-      pub = total - ((tid == pad_digit) ? (u32)(TILE - valid) : 0u);
-      if constexpr (!EARLY)
-        st_relaxed(lookback + (u64)tile * 256 + tid, (tile == 0 ? kLbInclusive : kLbPartial) | lb_epoch(epoch) | (u64)pub);
-      if constexpr (CDESC) {
-        if (tile > 0) cwin = ld_relaxed_v4(part + ((u64)((tile - 1) >> 2) * 256 + tid) * 4);  // up to 4 predecessors
-      } else {
+      pub = total - ((tid == 255) ? (u32)(TILE - valid) : 0u);
 #pragma unroll
-        for (int j = 0; j < LB1; ++j)
-          win[j] = (tile > (u32)j) ? ld_relaxed(lookback + (u64)(tile - 1 - j) * 256 + tid) : 0ull;
-      }
+      for (int j = 0; j < LBW; ++j)
+        win[j] = (tile > (u32)j) ? ld_relaxed(lookback + (u64)(tile - 1 - j) * 256 + tid) : 0ull;
       // counters become: position in the tile of the warp's first record with this digit
       u32 run = excl;
-      if constexpr (BATCH_P) {
-        constexpr int H = (NROW + 1) / 2;
 #pragma unroll
-        for (int h0 = 0; h0 < NROW; h0 += H) {
-          u32 c[H];
-#pragma unroll
-          for (int w = 0; w < H; ++w) c[w] = (h0 + w < NROW) ? s_cnt[((h0 + w) * 256 + tid) * CS + CO] : 0u;
-#pragma unroll
-          for (int w = 0; w < H; ++w)
-            if (h0 + w < NROW) {
-              s_cnt[((h0 + w) * 256 + tid) * CS + CO] = run;
-              run += c[w];
-            }
-        }
-      } else {
-#pragma unroll
-        for (int w = 0; w < NROW; ++w) {
-          const u32 c = s_cnt[(w * 256 + tid) * CS + CO];
-          s_cnt[(w * 256 + tid) * CS + CO] = run;
-          run += c;
-        }
+      for (int w = 0; w < NW; ++w) {
+        const u32 c = s_cnt[w * 256 + tid];
+        s_cnt[w * 256 + tid] = run;
+        run += c;
       }
     }
     __syncthreads();  // B3
     MHB_TL_MARK(3);
 
     // ---- reorder in shared memory: every digit's records become contiguous, input order kept ----
-    if constexpr (BATCH_R) {
 #pragma unroll
-      for (int i = 0; i < IPT; ++i) rk[i] = my_cnt[(i >= HA ? 256 : 0) + (rk[i] & 255u) * CS + CO] + (rk[i] >> 8);
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) st_shared_rec<WR>(s_recs, rk[i], r[i]);
-    } else {
-#pragma unroll
-      for (int i = 0; i < IPT; ++i) {
-        const u32 pos = my_cnt[(i >= HA ? 256 : 0) + (rk[i] & 255u) * CS + CO] + (rk[i] >> 8);
-        st_rec<WR>(s_recs, pos, r[i]);
-      }
+    for (int i = 0; i < IPT; ++i) {
+      const u32 pos = my_cnt[rk[i] & 255u] + (rk[i] >> 8);
+      st_rec<WR>(s_recs, pos, r[i]);
     }
     MHB_TL_MARK(4);
     const u32 next_tile = s_misc[0];  // written before B3, rewritten only after the next tile's B1
-    if constexpr (PREFETCH && !LATEPF) {
-      if (next_tile < num_tiles) load_tile(next_tile);
-    }
 
     // ---- global offsets by decoupled look-back.  All CTAs run the same phases almost in step, so the nearest
     // predecessors are still "partial" when a tile looks back and the walk to the last "inclusive" descriptor is long
-    // (profiles/r1b: 25 % of all warp samples were this loop + the CTA waiting for it at B4 when it fetched 2
-    // descriptors per L2 round trip).  After the two prefetched descriptors the walk therefore fetches LBW at a
-    // time - all loads in flight together, one round trip per LBW predecessors.
-    if constexpr (CDESC) {
-      if (tid < 256) {
-        u64 prefix = 0;
-        if (tile > 0) {
-          u32 tcur = tile - 1;  // the predecessor to account for next; cwin holds its group of four
-          uint4 cur = cwin;
-          while (true) {
-            const u32 e = tcur & 3u;
-            const u32 *gp = part + ((u64)(tcur >> 2) * 256 + tid) * 4;
-            u32 w = pick4(cur, e);
-            MHB_TL_DEPTH();
-            while ((w >> 30) == 0u || (w & (255u << 22)) != ep22) {  // not published yet (or a previous pass's word)
-              MHB_TL_SPIN();
-              cur = ld_relaxed_v4(gp);
-              w = pick4(cur, e);
-            }
-            if ((w >> 30) == 3u) {  // this tile's inclusive prefix exists: one 64-bit load ends the walk
-              const u64 *ip = lookback + (u64)tcur * 256 + tid;
-              u64 v = ld_relaxed(ip);
-              while ((v & kLbStatusMask) != kLbInclusive || (v & lb_epoch(255)) != lb_epoch(epoch)) v = ld_relaxed(ip);
-              prefix += v & kLbValueMask;
-              break;
-            }
-            prefix += w & 0x3FFFFFu;
-            if (tcur == 0) break;  // not reachable: tile 0 always carries status 3
-            --tcur;
-            if ((tcur & 3u) == 3u) cur = ld_relaxed_v4(part + ((u64)(tcur >> 2) * 256 + tid) * 4);  // next group of four
-          }
-          st_relaxed(lookback + (u64)tile * 256 + tid, kLbInclusive | lb_epoch(epoch) | (prefix + (u64)pub));
-          st_relaxed_u32(part + ((u64)(tile >> 2) * 256 + tid) * 4 + (tile & 3u), (3u << 30) | ep22 | pub);
-        }
-        s_glob[tid] = bin_addr[tid] + (prefix - (u64)excl) * (u64)(WR * 4);
-        MHB_TL_LB_DONE();
-        MHB_TL_MARK(5);
-      }
-    } else if (tid < 256) {
+    // (profiles/r1b: 25 % of all warp samples were this loop + the CTA waiting for it at B4).  The walk therefore
+    // fetches LBW descriptors at a time - all loads in flight together, one round trip per LBW predecessors; the first
+    // window was requested before the reorder.
+    if (tid < 256) {
       u64 prefix = 0;
       if (tile > 0) {
         const u64 epv = lb_epoch(epoch);
         u32 p = tile - 1;  // descriptor win[0] belongs to tile p
         bool done = false;
 #pragma unroll
-        for (int j = 0; j < LB1; ++j) {
+        for (int j = 0; j < LBW; ++j) {
           if (!done) {
             u64 v = win[j];
             const u64 *pp = lookback + (u64)(p - j) * 256 + tid;
@@ -539,7 +338,7 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
           }
         }
         while (!done) {
-          p -= LB1;
+          p -= LBW;
           u64 wv[LBW];
 #pragma unroll
           for (int j = 0; j < LBW; ++j)
@@ -558,8 +357,6 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
               if ((v & kLbStatusMask) == kLbInclusive || p == (u32)j) done = true;
             }
           }
-          p += (u32)LB1;
-          p -= (u32)LBW;  // so that the next `p -= LB1` lands LBW further back (p >= LBW here)
         }
         st_relaxed(lookback + (u64)tile * 256 + tid, kLbInclusive | epv | (prefix + (u64)pub));
       }
@@ -570,50 +367,22 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
     __syncthreads();  // B4: s_recs and s_glob complete; nobody reads the counters any more
     MHB_TL_MARK(6);
 
-    if constexpr (PREFETCH && LATEPF) {
-      if (next_tile < num_tiles) load_tile(next_tile);  // in flight during the scatter; does not delay the look-back
-    }
     // ---- coalesced scatter + next digit's histogram; clear the counters for the next tile ----
     {
       uint4 *z = reinterpret_cast<uint4 *>(s_cnt);
-      for (int i = tid; i < NROW * 256 * CS / 4; i += THREADS) z[i] = make_uint4(0u, 0u, 0u, 0u);
-      if constexpr (EARLY)
-        for (int i = tid; i < 256; i += THREADS) s_early[i] = 0;
+      for (int i = tid; i < NW * 256 / 4; i += THREADS) z[i] = make_uint4(0u, 0u, 0u, 0u);
+      for (int i = tid; i < 256; i += THREADS) s_early[i] = 0;
     }
     const u64 my_off = (u64)tid * (WR * 4);
-    if (full && !BATCH) {
+    if (full) {
 #pragma unroll
       for (int i = 0; i < IPT; ++i) {
         const u32 p = (u32)i * THREADS + tid;
         u32 q[WR];
         ld_rec<WR>(s_recs, p, q);
-        u32 dd = rec_digit<WR>(q, widx, bsel);
-        if constexpr (OWNER_LUT) dd = s_lut[dd];
+        const u32 dd = rec_digit<WR>(q, widx, bsel);
         st_rec<WR>(reinterpret_cast<u32 *>(s_glob[dd] + my_off + (u64)i * (THREADS * WR * 4)), 0, q);
         if constexpr (HAS_NEXT) atomicAdd(&s_next[rec_digit<WR>(q, nwidx, nbsel)], 1u);
-      }
-    } else if (full) {
-      constexpr int CH = PREFETCH ? 4 : (WR <= 2 ? 6 : (WR <= 4 ? 4 : 2));  // records whose loads are issued together
-#pragma unroll
-      for (int c0 = 0; c0 < IPT; c0 += CH) {
-        u32 q[CH][WR];
-        u64 g[CH];
-#pragma unroll
-        for (int j = 0; j < CH; ++j)
-          if (c0 + j < IPT) ld_rec<WR>(s_recs, (u32)(c0 + j) * THREADS + tid, q[j]);
-#pragma unroll
-        for (int j = 0; j < CH; ++j)
-          if (c0 + j < IPT) {
-            u32 dd = rec_digit<WR>(q[j], widx, bsel);
-            if constexpr (OWNER_LUT) dd = s_lut[dd];
-            g[j] = s_glob[dd];
-          }
-#pragma unroll
-        for (int j = 0; j < CH; ++j)
-          if (c0 + j < IPT) {
-            st_global_rec<WR>(g[j] + my_off + (u64)(c0 + j) * (THREADS * WR * 4), q[j]);
-            if constexpr (HAS_NEXT) red_shared_inc(&s_next[rec_digit<WR>(q[j], nwidx, nbsel)]);
-          }
       }
     } else {
 #pragma unroll
@@ -622,8 +391,7 @@ __global__ void __launch_bounds__(SortCfg3<WR, CFG>::THREADS, SortCfg3<WR, CFG>:
         if (p < valid) {
           u32 q[WR];
           ld_rec<WR>(s_recs, p, q);
-          u32 dd = rec_digit<WR>(q, widx, bsel);
-          if constexpr (OWNER_LUT) dd = s_lut[dd];
+          const u32 dd = rec_digit<WR>(q, widx, bsel);
           st_rec<WR>(reinterpret_cast<u32 *>(s_glob[dd] + (u64)p * (WR * 4)), 0, q);
           if constexpr (HAS_NEXT) atomicAdd(&s_next[rec_digit<WR>(q, nwidx, nbsel)], 1u);
         }

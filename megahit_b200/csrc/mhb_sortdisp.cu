@@ -1,7 +1,7 @@
-// mhb_sortdisp.cu -- the radix-sort part of the device-level C ABI (include/mhb.h, layer 1): variant selection,
-// per-width dispatch of the radix pass kernels (mhb_sort.cuh v2 = partition pass, mhb_sort3.cuh v3 = sort passes),
-// the fused partition + exchange pass, CUDA-IPC buffer helpers and the per-pass timing trace.  Its own translation
-// unit because the kernel instantiations (17 record widths x variants) dominate the build time of the library.
+// mhb_sortdisp.cu -- the radix-sort part of the device-level C ABI (include/mhb.h, layer 1): per-width dispatch of the
+// radix pass kernels (mhb_sort3.cuh = stable sort pass, mhb_part.cuh = unstable first pass and exchange pass), the
+// fused partition + exchange pass, CUDA-IPC buffer helpers and the per-pass timing trace.  Its own translation unit
+// because the kernel instantiations (17 record widths) dominate the build time of the library.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -19,63 +19,9 @@ using namespace mhb;
 // ------------------------------------------------------------------------------------------------
 // sort
 // ------------------------------------------------------------------------------------------------
-// Radix-pass variants.  0..3 = v2 geometries (mhb_sort.cuh); 256 + bits = v3 (mhb_sort3.cuh, see SortCfg3 for the
-// bit field).  Only the listed v3 combinations are instantiated (all for 8- and 12-byte records, the first one for
-// every record width).
-#define MHB_V3_DEFAULT 0x080
-#define MHB_V3_LIST(X) X(0x080) X(0x000) X(0x180) X(0x1080) X(0x082)
-static bool v3_listed(int bits) {
-#define X(B) \
-  if (bits == B) return true;
-  MHB_V3_LIST(X)
-#undef X
-  return false;
-}
-static int g_sort_cfg = -1;
-extern "C" int mhb_set_sort_cfg(int cfg) {
-  if (!((cfg >= 0 && cfg <= 3) || (cfg >= 256 && v3_listed(cfg - 256))))
-    return mhb_set_error(MHB_ERR_ARG, "unknown sort configuration %d", cfg);
-  g_sort_cfg = cfg;
-  return MHB_OK;
-}
-static int sort_cfg() {
-  int &cfg = g_sort_cfg;
-  if (cfg < 0) {
-    const char *e = getenv("MHB_SORT_CFG");
-    cfg = e ? atoi(e) : 256 + MHB_V3_DEFAULT;
-    if (!((cfg >= 0 && cfg <= 3) || (cfg >= 256 && v3_listed(cfg - 256)))) cfg = 256 + MHB_V3_DEFAULT;
-  }
-  return cfg;
-}
-template <int WR, int CFG>
-static u64 sort_tiles_cfg(u64 n) {
-  return (n + SortCfg<WR, CFG>::TILE - 1) / SortCfg<WR, CFG>::TILE;
-}
-template <int WR, int CFG>
-static u64 sort_tiles_cfg3(u64 n) {
-  return (n + SortCfg3<WR, CFG>::TILE - 1) / SortCfg3<WR, CFG>::TILE;
-}
 template <int WR>
 static u64 sort_tiles(u64 n) {
-  const int cfg = sort_cfg();
-  if (cfg >= 256) {
-    if constexpr (WR == 2 || WR == 3) {
-#define X(B) \
-  if (cfg - 256 == B) return sort_tiles_cfg3<WR, B>(n);
-      MHB_V3_LIST(X)
-#undef X
-    }
-    return sort_tiles_cfg3<WR, MHB_V3_DEFAULT>(n);
-  }
-  if constexpr (WR <= 3) {
-    switch (cfg) {
-      case 1: return sort_tiles_cfg<WR, 1>(n);
-      case 2: return sort_tiles_cfg<WR, 2>(n);
-      case 3: return sort_tiles_cfg<WR, 3>(n);
-      default: break;
-    }
-  }
-  return sort_tiles_cfg<WR, 0>(n);
+  return (n + SortCfg3<WR>::TILE - 1) / SortCfg3<WR>::TILE;
 }
 static u64 sort_num_tiles(u64 n, u32 words) {
 #define M(WW) \
@@ -85,123 +31,64 @@ static u64 sort_num_tiles(u64 n, u32 words) {
   return 0;
 }
 static constexpr size_t kSortHeadBytes = (size_t)(72 + 1) * 256 * 8 /*hist*/ + 256 * 8 /*bin_base*/ + 128 * 4 + 256 * 8 /*gcursor*/;
-// look-back storage for `tiles` tiles: 256 64-bit descriptors per tile + (compact-descriptor variants) one 16-byte
-// word per digit and group of four tiles behind them
-static size_t lb_bytes(u64 tiles) { return (size_t)tiles * 256 * 8 + (size_t)((tiles + 3) / 4) * 256 * 16; }
 
+// head + the look-back descriptors of the stable pass: 256 64-bit descriptors per tile
 extern "C" size_t mhb_sort_workspace_bytes(uint64_t n, uint32_t words) {
-  // sized for the smallest tile of any configuration so that a workspace stays valid across MHB_SORT_CFG values
-  u64 tiles = sort_num_tiles(n, words);
-  if (words <= 3) tiles = (n + 256 * 8 - 1) / (256 * 8) > tiles ? (n + 256 * 8 - 1) / (256 * 8) : tiles;
-#define M(WW) \
-  if (words == WW && sort_tiles_cfg<WW, 0>(n) > tiles) tiles = sort_tiles_cfg<WW, 0>(n);  // partition pass geometry
-  MHB_FOR_WR(M)
-#undef M
-  return kSortHeadBytes + lb_bytes(tiles) + 256;
+  return kSortHeadBytes + (size_t)sort_num_tiles(n, words) * 256 * 8 + 256;
 }
 
-template <int WR, int CFG>
-static int launch_radix_pass_cfg(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_base,
-                                 u64 *lookback, u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch) {
-  using C = SortCfg<WR, CFG>;
+template <int WR>
+static int launch_radix_pass(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_base, u64 *lookback,
+                             u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch) {
+  using C = SortCfg3<WR>;
   static int blocks_per_sm = 0;
   if (!blocks_per_sm) {
-    CK(cudaFuncSetAttribute(k_radix_pass<WR, CFG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_radix_pass<WR, CFG>, C::THREADS, C::SMEM));
+    CK(cudaFuncSetAttribute(k_radix_pass3<WR, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
+    CK(cudaFuncSetAttribute(k_radix_pass3<WR, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_radix_pass3<WR, true>, C::THREADS, C::SMEM));
     if (blocks_per_sm < 1) return mhb_set_error(MHB_ERR_CUDA, "radix pass kernel (WR=%d) does not fit an SM", WR);
-    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] radix pass WR=%d cfg=%d: %d threads x %d rec, %zu B smem, %d CTA/SM\n", WR, CFG, C::THREADS, C::IPT, C::SMEM, blocks_per_sm);
+    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] radix pass WR=%d: %d threads x %d rec, %zu B smem, %d CTA/SM\n", WR, C::THREADS, C::IPT, C::SMEM, blocks_per_sm);
   }
-  const u64 tiles = sort_tiles_cfg<WR, CFG>(n);
-  u64 grid = (u64)blocks_per_sm * sm_count();
-  if (grid > tiles) grid = tiles;
-  k_radix_pass<WR, CFG><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, lookback,
-                                                                 tile_counter, next_hist, next_byte, epoch);
-  CK_LAUNCH();
-  return MHB_OK;
-}
-
-template <int WR, int CFG>
-static int launch_radix_pass_cfg3(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_base,
-                                  u64 *lookback, u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch) {
-  using C = SortCfg3<WR, CFG>;
-  static int blocks_per_sm = 0;
-  if (!blocks_per_sm) {
-    CK(cudaFuncSetAttribute(k_radix_pass3<WR, CFG, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaFuncSetAttribute(k_radix_pass3<WR, CFG, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_radix_pass3<WR, CFG, false, true>, C::THREADS, C::SMEM));
-    if (blocks_per_sm < 1) return mhb_set_error(MHB_ERR_CUDA, "radix pass v3 kernel (WR=%d) does not fit an SM", WR);
-    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] radix pass v3 WR=%d bits=0x%03x: %d threads x %d rec, rank %d, prefetch %d, look-back %d/%d, batch %d, early %d, %zu B smem, %d CTA/SM\n", WR, CFG, C::THREADS, C::IPT, C::RANK, (int)C::PREFETCH, C::LB1, C::LBW, (int)C::BATCH, (int)C::EARLY, C::SMEM, blocks_per_sm);
-  }
-  const u64 tiles = sort_tiles_cfg3<WR, CFG>(n);
+  const u64 tiles = sort_tiles<WR>(n);
   u64 grid = (u64)blocks_per_sm * sm_count();
   if (grid > tiles) grid = tiles;
   if (next_hist)
-    k_radix_pass3<WR, CFG, false, true><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, lookback,
-                                                                                 tile_counter, next_hist, next_byte, epoch);
+    k_radix_pass3<WR, true><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, lookback, tile_counter,
+                                                                    next_hist, next_byte, epoch);
   else
-    k_radix_pass3<WR, CFG, false, false><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, lookback,
-                                                                                  tile_counter, nullptr, 0, epoch);
+    k_radix_pass3<WR, false><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, lookback, tile_counter,
+                                                                     nullptr, 0, epoch);
   CK_LAUNCH();
   return MHB_OK;
 }
 
-// first pass of a sort whose caller does not need a deterministic order among fully equal keys (mhb_part.cuh)
-template <int WR>
+// unstable pass (mhb_part.cuh): the first pass of a sort whose caller does not need a deterministic order among fully
+// equal keys (OWNER_LUT = false), and the exchange pass, whose digit is the owning rank (OWNER_LUT = true)
+template <int WR, bool OWNER_LUT>
 static int launch_part_unstable(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_base,
                                 unsigned long long *gcursor, u32 *tile_counter, u64 *next_hist, int next_byte,
                                 const uint8_t *lut) {
   using C = PartCfg<WR>;
+  constexpr size_t SMEM_HIST = OWNER_LUT ? C::SMEM_OWNER_HIST : C::SMEM;
   static int bps = 0;
   if (!bps) {
-    CK(cudaFuncSetAttribute(k_part_unstable<WR, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaFuncSetAttribute(k_part_unstable<WR, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaFuncSetAttribute(k_part_unstable<WR, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaFuncSetAttribute(k_part_unstable<WR, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_OWNER_HIST));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_part_unstable<WR, false, true>, C::THREADS, C::SMEM));
+    CK(cudaFuncSetAttribute(k_part_unstable<WR, OWNER_LUT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_HIST));
+    CK(cudaFuncSetAttribute(k_part_unstable<WR, OWNER_LUT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_part_unstable<WR, OWNER_LUT, true>, C::THREADS, SMEM_HIST));
     if (bps < 1) return mhb_set_error(MHB_ERR_CUDA, "partition pass (WR=%d) does not fit an SM", WR);
-    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] unstable partition pass WR=%d: %d threads x %d rec, %zu B smem, %d CTA/SM\n", WR, C::THREADS, C::IPT, C::SMEM, bps);
+    if (getenv("MHB_VERBOSE")) fprintf(stderr, "[mhb] unstable partition pass WR=%d owner=%d: %d threads x %d rec, %zu B smem, %d CTA/SM\n", WR, (int)OWNER_LUT, C::THREADS, C::IPT, SMEM_HIST, bps);
   }
   const u64 tiles = (n + C::TILE - 1) / C::TILE;
   u64 grid = (u64)bps * sm_count();
   if (grid > tiles) grid = tiles;
-  if (lut && next_hist)
-    k_part_unstable<WR, true, true><<<(int)grid, C::THREADS, C::SMEM_OWNER_HIST, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
-                                                                                       tile_counter, next_hist, next_byte, lut);
-  else if (lut)
-    k_part_unstable<WR, true, false><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
-                                                                             tile_counter, nullptr, 0, lut);
-  else if (next_hist)
-    k_part_unstable<WR, false, true><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
-                                                                             tile_counter, next_hist, next_byte, nullptr);
+  if (next_hist)
+    k_part_unstable<WR, OWNER_LUT, true><<<(int)grid, C::THREADS, SMEM_HIST, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
+                                                                                   tile_counter, next_hist, next_byte, lut);
   else
-    k_part_unstable<WR, false, false><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
-                                                                              tile_counter, nullptr, 0, nullptr);
+    k_part_unstable<WR, OWNER_LUT, false><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_base, gcursor,
+                                                                                  tile_counter, nullptr, 0, lut);
   CK_LAUNCH();
   return MHB_OK;
-}
-
-template <int WR>
-static int launch_radix_pass(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_base,
-                             u64 *lookback, u32 *tile_counter, u64 *next_hist, int next_byte, u32 epoch) {
-  const int cfg = sort_cfg();
-  if (cfg >= 256) {
-    if constexpr (WR == 2 || WR == 3) {
-#define X(B) \
-  if (cfg - 256 == B) return launch_radix_pass_cfg3<WR, B>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
-      MHB_V3_LIST(X)
-#undef X
-    }
-    return launch_radix_pass_cfg3<WR, MHB_V3_DEFAULT>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
-  }
-  if constexpr (WR <= 3) {
-    switch (cfg) {
-      case 1: return launch_radix_pass_cfg<WR, 1>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
-      case 2: return launch_radix_pass_cfg<WR, 2>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
-      case 3: return launch_radix_pass_cfg<WR, 3>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
-      default: break;
-    }
-  }
-  return launch_radix_pass_cfg<WR, 0>(st, in, n, byte_idx, bin_base, lookback, tile_counter, next_hist, next_byte, epoch);
 }
 
 #ifdef MHB_SORT_TIMELINE
@@ -228,7 +115,7 @@ uint64_t g_trace_seq = 0;
 }  // namespace
 
 // relaxed != 0: the first pass may be the unstable partition pass (mhb_part.cuh) - the order among records whose sorted
-// bytes are ALL equal is then unspecified; MHB_SORT_STABLE_FIRST=1 keeps the stable pass everywhere (A/B hook)
+// bytes are ALL equal is then unspecified
 int mhb_sort_records_ex(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint32_t words, const uint8_t *bytes,
                         uint32_t n_bytes, const uint64_t *first_hist, void *ws, size_t ws_bytes, int *result_in_b,
                         double *pass_ms_host, int relaxed);
@@ -241,8 +128,6 @@ int mhb_sort_records_impl(void *stream, uint32_t *a, uint32_t *b, uint64_t n, ui
 int mhb_sort_records_ex(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint32_t words, const uint8_t *bytes,
                           uint32_t n_bytes, const uint64_t *first_hist, void *ws, size_t ws_bytes, int *result_in_b,
                         double *pass_ms_host, int relaxed) {
-  static const bool stable_first = getenv("MHB_SORT_STABLE_FIRST") != nullptr;
-  if (stable_first) relaxed = 0;
   if (words < 1 || words > 17 || n_bytes > 72 || !result_in_b)
     return mhb_set_error(MHB_ERR_ARG, "bad sort geometry (words=%u n_bytes=%u)", words, n_bytes);
   *result_in_b = 0;
@@ -255,8 +140,7 @@ int mhb_sort_records_ex(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint
   u32 *tile_counter = (u32 *)(bin_base + 256);  // [128]
   unsigned long long *gcursor = (unsigned long long *)(tile_counter + 128);  // [256]: unstable first pass
   u64 *lookback = (u64 *)((char *)ws + kSortHeadBytes);
-  // only what this sort's tile geometry touches (the workspace itself is sized for the smallest tile of any variant)
-  CK(cudaMemsetAsync(ws, 0, kSortHeadBytes + lb_bytes(sort_num_tiles(n, words)) + 256, st));
+  CK(cudaMemsetAsync(ws, 0, mhb_sort_workspace_bytes(n, words), st));
   if (first_hist) {
     CK(cudaMemcpyAsync(hist, first_hist, 256 * 8, cudaMemcpyDeviceToDevice, st));
   } else {
@@ -282,8 +166,8 @@ int mhb_sort_records_ex(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint
     u64 *next_hist = p + 1 < n_bytes ? hist + (u64)(p + 1) * 256 : nullptr;
     const int next_byte = p + 1 < n_bytes ? bytes[p + 1] : 0;
     int rc = MHB_ERR_ARG;
-    if (p == 0 && relaxed && words == 2) rc = launch_part_unstable<2>(st, in, n, bytes[p], bin_base, gcursor, tile_counter + p, next_hist, next_byte, nullptr);
-    else if (p == 0 && relaxed && words == 3) rc = launch_part_unstable<3>(st, in, n, bytes[p], bin_base, gcursor, tile_counter + p, next_hist, next_byte, nullptr);
+    if (p == 0 && relaxed && words == 2) rc = launch_part_unstable<2, false>(st, in, n, bytes[p], bin_base, gcursor, tile_counter + p, next_hist, next_byte, nullptr);
+    else if (p == 0 && relaxed && words == 3) rc = launch_part_unstable<3, false>(st, in, n, bytes[p], bin_base, gcursor, tile_counter + p, next_hist, next_byte, nullptr);
     else {
 #define M(WW) \
   if (words == WW) rc = launch_radix_pass<WW>(st, in, n, bytes[p], bin_base, lookback, tile_counter + p, next_hist, next_byte, p + 1);
@@ -311,82 +195,45 @@ int mhb_sort_records_ex(void *stream, uint32_t *a, uint32_t *b, uint64_t n, uint
 // ------------------------------------------------------------------------------------------------
 // fused partition + exchange: one radix pass whose per-digit destinations are arbitrary device addresses, e.g.
 // slots inside OTHER GPUs' receive buffers opened through CUDA IPC.  The scatter stores travel over NVLink while
-// the rest of the tile is still being ranked - no separate all-to-all.
+// the rest of the tile is still being ranked - no separate all-to-all.  The exchange has no earlier order to preserve
+// (every receiving stage re-sorts and tallies, or takes the minimum over equal keys), so it is the unstable pass.
 // ------------------------------------------------------------------------------------------------
-template <int WR>
-static int launch_partition_pass(cudaStream_t st, const u32 *in, u64 n, int byte_idx, const u64 *bin_addr, u64 *lookback,
-                                 u32 *tile_counter, const uint8_t *lut) {
-  using C = SortCfg<WR, 0>;
-  static int blocks_per_sm = 0;
-  if (!blocks_per_sm) {
-    CK(cudaFuncSetAttribute(k_radix_pass<WR, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_radix_pass<WR, 0, true>, C::THREADS, C::SMEM));
-    if (blocks_per_sm < 1) return mhb_set_error(MHB_ERR_CUDA, "partition pass kernel (WR=%d) does not fit an SM", WR);
-  }
-  const u64 tiles = sort_tiles_cfg<WR, 0>(n);
-  u64 grid = (u64)blocks_per_sm * sm_count();
-  if (grid > tiles) grid = tiles;
-  k_radix_pass<WR, 0, true><<<(int)grid, C::THREADS, C::SMEM, st>>>(in, n, (u32)tiles, byte_idx, bin_addr, lookback,
-                                                                     tile_counter, nullptr, 0, 1, lut);
-  CK_LAUNCH();
-  return MHB_OK;
-}
-
 static int partition_scatter_impl(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
                                   const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws, size_t ws_bytes,
-                                  int next_byte, uint64_t *owner_next_hist, int *hist_done);
+                                  int next_byte, uint64_t *owner_next_hist) {
+  if (!owner_of_byte_dev) return mhb_set_error(MHB_ERR_ARG, "owner table is NULL");
+  if (words < 1 || words > 17 || byte < 0 || byte >= (int)(4 * words)) return mhb_set_error(MHB_ERR_ARG, "bad geometry");
+  if (n == 0) return MHB_OK;
+  if (ws_bytes < kSortHeadBytes) return mhb_set_error(MHB_ERR_ARG, "sort workspace too small");
+  cudaStream_t st = (cudaStream_t)stream;
+  u32 *tile_counter = (u32 *)((u64 *)ws + (72 + 1) * 256 + 256);
+  unsigned long long *gcursor = (unsigned long long *)(tile_counter + 128);
+  CK(cudaMemsetAsync(ws, 0, kSortHeadBytes, st));
+  int rc = MHB_ERR_ARG;
+#define M(WW)                                                                                                          \
+  if (words == WW)                                                                                                     \
+    rc = launch_part_unstable<WW, true>(st, recs, n, byte, bin_addr_dev, gcursor, tile_counter, owner_next_hist, next_byte, \
+                                        owner_of_byte_dev);
+  MHB_FOR_WR(M)
+#undef M
+  return rc;
+}
 extern "C" int mhb_partition_scatter(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
                                      const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws,
                                      size_t ws_bytes) {
-  return partition_scatter_impl(stream, recs, n, words, byte, owner_of_byte_dev, bin_addr_dev, ws, ws_bytes, 0, nullptr, nullptr);
+  return partition_scatter_impl(stream, recs, n, words, byte, owner_of_byte_dev, bin_addr_dev, ws, ws_bytes, 0, nullptr);
 }
 extern "C" int mhb_partition_scatter_hist(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
                                           const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws,
                                           size_t ws_bytes, int next_byte, uint64_t *owner_next_hist, int *hist_done) {
   if (!owner_of_byte_dev || !owner_next_hist || !hist_done || next_byte < 0 || next_byte >= (int)(4 * words))
     return mhb_set_error(MHB_ERR_ARG, "bad owner-histogram arguments");
-  return partition_scatter_impl(stream, recs, n, words, byte, owner_of_byte_dev, bin_addr_dev, ws, ws_bytes, next_byte,
-                                owner_next_hist, hist_done);
-}
-static int partition_scatter_impl(void *stream, const uint32_t *recs, uint64_t n, uint32_t words, int byte,
-                                  const uint8_t *owner_of_byte_dev, const uint64_t *bin_addr_dev, void *ws, size_t ws_bytes,
-                                  int next_byte, uint64_t *owner_next_hist, int *hist_done) {
-  if (hist_done) *hist_done = 0;
-  if (words < 1 || words > 17 || byte < 0 || byte >= (int)(4 * words)) return mhb_set_error(MHB_ERR_ARG, "bad geometry");
-  if (n == 0) return MHB_OK;
-  // the partition pass always runs the v2 kernel in geometry 0, whatever variant the sorts use
-  u64 tiles = 0;
-#define M(WW) \
-  if (words == WW) tiles = sort_tiles_cfg<WW, 0>(n);
-  MHB_FOR_WR(M)
-#undef M
-  const size_t need = kSortHeadBytes + (size_t)tiles * 256 * 8 + 256;
-  if (ws_bytes < need) return mhb_set_error(MHB_ERR_ARG, "sort workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
-  u64 *hist = (u64 *)ws;
-  u32 *tile_counter = (u32 *)(hist + (72 + 1) * 256 + 256);
-  u64 *lookback = (u64 *)((char *)ws + kSortHeadBytes);
-  CK(cudaMemsetAsync(ws, 0, need, st));
-  int rc = MHB_ERR_ARG;
-  static const bool stable_first = getenv("MHB_SORT_STABLE_FIRST") != nullptr;
-  if (owner_of_byte_dev && !stable_first && (words == 2 || words == 3)) {
-    // the exchange has no earlier order to preserve: unstable pass (no look-back chain), 8- and 12-byte records
-    unsigned long long *gcursor = (unsigned long long *)(tile_counter + 128);
-    rc = words == 2 ? launch_part_unstable<2>(st, recs, n, byte, bin_addr_dev, gcursor, tile_counter, owner_next_hist, next_byte, owner_of_byte_dev)
-                    : launch_part_unstable<3>(st, recs, n, byte, bin_addr_dev, gcursor, tile_counter, owner_next_hist, next_byte, owner_of_byte_dev);
-    if (!rc && owner_next_hist && hist_done) *hist_done = 1;
-  } else if (owner_of_byte_dev) {
-#define M(WW) \
-  if (words == WW) rc = launch_partition_pass<WW>(st, recs, n, byte, bin_addr_dev, lookback, tile_counter, owner_of_byte_dev);
-    MHB_FOR_WR(M)
-#undef M
-  } else {
-#define M(WW) \
-  if (words == WW) rc = launch_radix_pass_cfg<WW, 0>(st, recs, n, byte, bin_addr_dev, lookback, tile_counter, nullptr, 0, 1);
-    MHB_FOR_WR(M)
-#undef M
-  }
-  return rc;
+  *hist_done = 0;
+  if (int rc = partition_scatter_impl(stream, recs, n, words, byte, owner_of_byte_dev, bin_addr_dev, ws, ws_bytes, next_byte,
+                                      owner_next_hist))
+    return rc;
+  *hist_done = 1;
+  return MHB_OK;
 }
 
 extern "C" int mhb_dev_malloc(void **ptr, size_t bytes) {

@@ -123,7 +123,7 @@ class IterateOpts(C.Structure):
 SYMBOLS = [
     "mhb_last_error", "mhb_version", "mhb_device_count", "mhb_launch_count", "mhb_count_record_words", "mhb_words_per_edge",
     "mhb_s2s_record_words", "mhb_count_sort_bytes", "mhb_s2s_sort_bytes", "mhb_sort_workspace_bytes",
-    "mhb_count_extract", "mhb_check_fixed_len", "mhb_count_extract_range", "mhb_set_round_limit", "mhb_set_s2s_round_limit", "mhb_plan_rounds", "mhb_plan_rounds16", "mhb_sort_records", "mhb_sort_records_relaxed", "mhb_sort_pass_ms", "mhb_set_sort_cfg", "mhb_partition_scatter", "mhb_partition_scatter_hist", "mhb_plan_partition", "mhb_compact_tip_edges", "mhb_dev_malloc", "mhb_dev_free",
+    "mhb_count_extract", "mhb_check_fixed_len", "mhb_count_extract_range", "mhb_set_round_limit", "mhb_set_s2s_round_limit", "mhb_plan_rounds", "mhb_plan_rounds16", "mhb_sort_records", "mhb_sort_records_relaxed", "mhb_sort_pass_ms", "mhb_partition_scatter", "mhb_partition_scatter_hist", "mhb_plan_partition", "mhb_compact_tip_edges", "mhb_dev_malloc", "mhb_dev_free",
     "mhb_ipc_export", "mhb_ipc_open", "mhb_ipc_close", "mhb_count_solid_scratch_bytes", "mhb_count_solid", "mhb_count_hashed_supported", "mhb_count_hashed_workspace_bytes", "mhb_count_solid_hashed", "mhb_tipset_bytes",
     "mhb_tipset_build", "mhb_count_mark_mercy", "mhb_count_tip_edges", "mhb_s2s_extract", "mhb_s2s_extract_range",
     "mhb_s2s_emit_scratch_bytes", "mhb_s2s_emit", "mhb_set_device", "mhb_count_host", "mhb_s2s_host", "mhb_build_host", "mhb_free",

@@ -187,9 +187,9 @@ class MultiGpuBuild:
         """Move every record to the rank owning its leading byte.  Fused mode: ONE kernel does partition + exchange -
         the radix pass's scatter stores go straight into the owners' receive buffers over NVLink (CUDA IPC peer
         pointers).  Fallback (MHB_MGPU_NCCL_A2A=1): local pass, then one variable-size NCCL all-to-all.
-        next_byte: the byte the owner's sort visits first - where the exchange pass supports it, it also counts that byte
-        per owner, the ranks swap the 256-bin rows, and self._first_hist (device int64[256], else None) is the
-        first-pass histogram of the owned records: the owner's sort need not sweep them to count.
+        next_byte: the byte the owner's sort visits first - the fused exchange pass also counts that byte per owner, the
+        ranks swap the 256-bin rows, and self._first_hist (device int64[256]; None on the fallback path or without
+        next_byte) is the first-pass histogram of the owned records: the owner's sort need not sweep them to count.
         Returns (pointer to the owned records, count, bounds[world+1] numpy, owner table numpy uint8[256])."""
         L, W = self.L, self.world
         rb = words * 4
@@ -246,8 +246,7 @@ class MultiGpuBuild:
         # row o of my table goes to rank o; the all-to-all is also the barrier after the scatter
         got = self._buf(tag + "_ohist_in", W * 256, torch.int64)[: W * 256]
         dist.all_to_all_single(got, oh[: W * 256])
-        if done.value:
-            self._first_hist = got.view(W, 256).sum(0).contiguous()
+        self._first_hist = got.view(W, 256).sum(0).contiguous()
         return pb.ptr, n_own, bounds, owner
 
     def close(self):

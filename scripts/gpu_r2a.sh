@@ -1,7 +1,7 @@
 #!/bin/bash
 # Round 2, GPU call A: strict GPU suite (incl. bench-scale parity vs the reference binary and downstream acceptance),
-# radix-pass variant sweep, vendor onesweep yardstick, bench with each opt-in switch, launch list + section-level ncu of
-# the non-sort kernels at bench size.
+# vendor onesweep yardstick, bench with the opt-in switch, launch list + section-level ncu of the non-sort kernels at
+# bench size.
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,clocks.max.sm,clocks.max.mem,power.limit --format=csv > gpurun_out/gpu_info.txt 2>&1
@@ -10,16 +10,6 @@ echo "== pytest -m gpu"
 timeout 1200 python -m pytest tests -m gpu -q --timeout 900 -rxXf > gpurun_out/pytest_gpu.log 2>&1; echo "pytest rc=$?"; tail -30 gpurun_out/pytest_gpu.log
 echo "== cub yardstick"
 timeout 120 scripts/diag/cub_yardstick.bin 1230000000 2>&1 | tee gpurun_out/cub_yardstick.jsonl
-echo "== radix-pass sweep"
-timeout 500 python scripts/sort_sweep.py 2> gpurun_out/sweep.err > gpurun_out/sweep.log
-python - <<PY
-import json
-for r in json.load(open('gpurun_out/sort_sweep.json')):
-    if 'wr2_pass_ms' in r:
-        print('cfg %6d (0x%05x) ok=%s wr2 %.2f ms  const %.2f  wr3 %.2f ms' % (r['cfg'], max(0, r['cfg'] - 256), r['ok'], sum(r['wr2_pass_ms']) / 7, min(r.get('wr2_const_digit_pass_ms', [0])), sum(r['wr3_pass_ms']) / 10))
-    else:
-        print(r)
-PY
 summ() { python - "$1" <<PY
 import json, sys
 try:
@@ -33,13 +23,8 @@ PY
 }
 echo "== bench: default (with cpu baseline)"
 timeout 400 python bench.py --steps 3 --warmup 3 > gpurun_out/bench_default.json 2> gpurun_out/bench_default.err; summ gpurun_out/bench_default.json
-echo "== bench: MHB_EXTRACT_ROLL=1"
-MHB_EXTRACT_ROLL=1 timeout 300 python bench.py --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/bench_roll.json 2> gpurun_out/bench_roll.err; summ gpurun_out/bench_roll.json
 echo "== bench: MHB_H2D_CHUNKS=4"
 MHB_H2D_CHUNKS=4 timeout 300 python bench.py --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/bench_chunks.json 2> gpurun_out/bench_chunks.err; summ gpurun_out/bench_chunks.json
-BEST=$(cat gpurun_out/best_cfg 2>/dev/null || echo 384)
-echo "== bench: best sort variant $BEST"
-MHB_SORT_CFG=$BEST timeout 300 python bench.py --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/bench_best.json 2> gpurun_out/bench_best.err; summ gpurun_out/bench_best.json
 echo "== ncu launch list at bench size"
 timeout 500 ncu --metrics gpu__time_duration.sum --clock-control none -c 600 --csv --log-file gpurun_out/launches_r2a_10M.csv \
    python bench.py --steps 1 --warmup 1 --no-cpu-baseline --e2e-steps 0 > gpurun_out/ncu_list.log 2>&1; echo rc=$?

@@ -1,11 +1,12 @@
 #!/usr/bin/env python
 """Per-tile timeline of one radix pass (diagnostic build: `make -C megahit_b200/csrc timeline`).
 
-    MHB_LIB=megahit_b200/libmhb_timeline.so python scripts/sort_timeline.py [n_records] [cfg] [words]
+    MHB_LIB=megahit_b200/libmhb_timeline.so python scripts/sort_timeline.py [n_records] [words] [rows.npy]
 
 Prints, for one pass over n random records: duration of every phase of a tile (us: median / p90 / max), the
 look-back depth and re-poll statistics, the stagger between consecutive tile starts, and how many tiles were in each
-phase at the moment a tile started its look-back.  Writes gpurun_out/sort_timeline_<cfg>.npy (rows x 16 uint64)."""
+phase at the moment a tile started its look-back.  With rows.npy, also saves a sample of the per-tile rows there
+(rows x 16 uint64)."""
 import ctypes as C
 import os
 import sys
@@ -19,11 +20,9 @@ os.environ.setdefault("MHB_LIB", os.path.join(ROOT, "megahit_b200", "libmhb_time
 from megahit_b200 import dev, lib  # noqa: E402
 
 n = int(float(sys.argv[1])) if len(sys.argv) > 1 else 1_230_000_000
-cfg = int(sys.argv[2], 0) if len(sys.argv) > 2 else 256 + 0x080
-words = int(sys.argv[3]) if len(sys.argv) > 3 else 2
+words = int(sys.argv[2]) if len(sys.argv) > 2 else 2
 L = lib.load()
 assert hasattr(L, "mhb_debug_set_sort_timeline"), "not the timeline build (MHB_LIB)"
-lib._check(L.mhb_set_sort_cfg(cfg))
 g = torch.Generator(device="cuda")
 g.manual_seed(3)
 a = torch.randint(-2**31, 2**31 - 1, (n * words + 4,), generator=g, device="cuda", dtype=torch.int32)
@@ -41,7 +40,7 @@ ms = lib.sort_pass_ms(0)[0]
 t = tl.cpu().numpy().view(np.uint64).reshape(rows, 16)
 t = t[t[:, 2] > 0]
 t = t[np.argsort(t[:, 0])]
-print(f"cfg {cfg} (0x{max(0, cfg - 256):04x}) words {words}: {len(t)} tiles, pass {ms[0]:.3f} ms "
+print(f"words {words}: {len(t)} tiles, pass {ms[0]:.3f} ms "
       f"({2 * n * words * 4 / (ms[0] * 1e-3) / 1e9:.0f} GB/s)")
 mhz = torch.cuda.get_device_properties(0).clock_rate / 1e3 if hasattr(torch.cuda.get_device_properties(0), "clock_rate") else 1965.0
 names = ["loads arrived", "early publish", "rank (B1)", "warp bases (B3)", "reorder", "look-back", "B4 passed", "scatter (B5)"]
@@ -75,5 +74,5 @@ for i in sample:
     depth_needed.append(i - j)
 print(f"distance to the nearest predecessor whose look-back had finished when a tile began its own: median "
       f"{np.median(depth_needed):.0f}, p90 {np.percentile(depth_needed, 90):.0f}")
-os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-np.save(os.path.join(ROOT, "gpurun_out", f"sort_timeline_{cfg}.npy"), t[:: max(1, len(t) // 20000)])
+if len(sys.argv) > 3:
+    np.save(sys.argv[3], t[:: max(1, len(t) // 20000)])

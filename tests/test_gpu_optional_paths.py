@@ -43,43 +43,6 @@ def test_fused_build_with_chunked_upload_matches_reference(name, k, m, gold):
         assert r["sdbg"] == gold["sdbg_sha256"] and r["edges"] == gold["edges_sha256"]
 
 
-# The new radix-pass variants (compact look-back descriptors, two-stream ranking) are deliberately NOT exercised here:
-# they contain spin-waits, and an unverified spin-wait does not belong in an unattended test run.  scripts/sort_sweep.py
-# checks and times them one process each, with a timeout (scripts/gpu_r2_first.sh).
-
-
-_CHILD_ROLL = r"""
-import json, os, sys
-import numpy as np
-sys.path.insert(0, %r)
-from megahit_b200 import formats as F, lib
-case, k, m = sys.argv[1], int(sys.argv[2]), int(sys.argv[3])
-bin_words = np.fromfile(os.path.join(case, "reads.lib.bin"), np.uint32)
-_, n_reads = F.read_lib_info(os.path.join(case, "reads.lib"))
-g = lib.count_host(bin_words, n_reads, k, m, want_mercy=True)
-print("RESULT " + json.dumps({"edges": F.sha256(g["edges"].tobytes()), "n_solid": int(g["n_solid"]),
-                              "cand": [int(x) for x in g["cand_ids"][:50]], "n_cand": int(len(g["cand_ids"])),
-                              "n_has_tips": int(g["n_has_tips"])}))
-""" % ROOT
-
-
-@pytest.mark.parametrize("name,k,m,gold", [c for c in golden_cases() if c.values[0] in ("syn150_k27", "synvar_k21_m3")])
-def test_rolling_extract_and_mark_match_default(name, k, m, gold):
-    """rolling record builder (MHB_EXTRACT_ROLL=1: extract and mercy-mark kernels; the mark kernel uses it by default) vs
-    the per-position kernels (MHB_EXTRACT_ROLL=0): same edges, same candidate reads, and those of the reference"""
-    import json
-    out = []
-    for roll in (False, True):
-        env = dict(os.environ, MHB_EXTRACT_ROLL="1" if roll else "0")
-        p = subprocess.run([sys.executable, "-c", _CHILD_ROLL, os.path.join(GOLDEN, name), str(k), str(m)], env=env,
-                           capture_output=True, text=True, timeout=300)
-        line = [l for l in p.stdout.splitlines() if l.startswith("RESULT ")]
-        assert line, p.stderr[-800:]
-        out.append(json.loads(line[-1][7:]))
-    assert out[0] == out[1]
-    assert out[1]["edges"] == gold["edges_sha256"] and out[1]["n_solid"] == gold["n_solid"]
-
-
 _CHILD_S2S = r"""
 import json, os, sys
 import numpy as np

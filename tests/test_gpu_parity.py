@@ -75,27 +75,23 @@ def test_sort_skewed_digits():
     assert (got == _np_lsd(recs, sort_bytes)).all()
 
 
-@pytest.mark.parametrize("cfg", [0, 1, 2, 3] + [256 + b for b in (0x080, 0x000, 0x082, 0x180, 0x1080)])
-def test_sort_every_pass_variant(cfg):
-    """every tile geometry / ranking variant of the radix pass (mhb_set_sort_cfg) gives the same stable LSD order,
-    including ragged last tiles and single-tile inputs"""
+@pytest.mark.parametrize("words,n,sort_bytes", [(2, 1, [1, 2, 3]), (2, 4607, [1, 2, 3, 4, 5, 6, 7]),
+                                                  (2, 6912 * 3 + 1, [1, 2, 3, 4, 5, 6, 7]), (2, 400_003, [1, 2, 3, 4, 5, 6, 7]),
+                                                  (3, 3071, [2, 5, 11]), (3, 200_001, [0, 1, 2, 4, 5, 6, 7, 8, 9, 10]),
+                                                  (4, 3840 * 2 + 1, [0, 6, 13]), (5, 30_011, [3, 9, 17]),
+                                                  (17, 768 * 5 + 7, [1, 40, 67])])
+def test_sort_ragged_and_single_tiles(words, n, sort_bytes):
+    """the stable LSD order with ragged last tiles and single-tile inputs (tiles of 6912, 4608, 3840, 2304 and 768
+    records at 2, 3, 4, 5 and 17 words)"""
     torch = _torch()
     from megahit_b200 import dev
-    L = lib.load()
-    lib._check(L.mhb_set_sort_cfg(cfg))
-    try:
-        rng = np.random.default_rng(cfg)
-        for words, n, sort_bytes in ((2, 1, [1, 2, 3]), (2, 4607, [1, 2, 3, 4, 5, 6, 7]), (2, 6912 * 3 + 1, [1, 2, 3, 4, 5, 6, 7]),
-                                     (2, 400_003, [1, 2, 3, 4, 5, 6, 7]), (3, 3071, [2, 5, 11]),
-                                     (3, 200_001, [0, 1, 2, 4, 5, 6, 7, 8, 9, 10]), (5, 30_011, [3, 9, 17])):
-            recs = rng.integers(0, 2 ** 32, size=(n, words), dtype=np.uint64).astype(np.uint32)
-            recs[:, 0] &= np.uint32(0x0F0F0F0F)
-            a = torch.from_numpy(np.concatenate([recs.view(np.int32).reshape(-1), np.zeros(4, np.int32)])).cuda()
-            out = dev.sort_records(a, torch.empty_like(a), n, words, sort_bytes)
-            got = out[: n * words].cpu().numpy().view(np.uint32).reshape(n, words)
-            assert (got == _np_lsd(recs, sort_bytes)).all(), (cfg, words, n)
-    finally:
-        lib._check(L.mhb_set_sort_cfg(int(os.environ.get("MHB_SORT_CFG", str(256 + 0x080)))))
+    rng = np.random.default_rng(words * 1_000_003 + n)
+    recs = rng.integers(0, 2 ** 32, size=(n, words), dtype=np.uint64).astype(np.uint32)
+    recs[:, 0] &= np.uint32(0x0F0F0F0F)
+    a = torch.from_numpy(np.concatenate([recs.view(np.int32).reshape(-1), np.zeros(4, np.int32)])).cuda()
+    out = dev.sort_records(a, torch.empty_like(a), n, words, sort_bytes)
+    got = out[: n * words].cpu().numpy().view(np.uint32).reshape(n, words)
+    assert (got == _np_lsd(recs, sort_bytes)).all()
 
 
 # ------------------------------------------------------------------------------------------------
